@@ -41,7 +41,8 @@ enum snacc_status {
 enum snacc_codec {
     SNACC_LZ4F = 0,    /* lz4framed.compress(b)   pairwise_ncd.py:80  (LZ4 frame, 64 KiB linked blocks) */
     SNACC_GZIP9 = 1,   /* gzip.compress(b)        pairwise_ncd.py:74  (deflate level 9, +18 wrapper)    */
-    SNACC_ZLIB6 = 2    /* zlib.compress(b)        pairwise_ncd.py:78  (deflate level 6, +6 wrapper)     */
+    SNACC_ZLIB6 = 2,   /* zlib.compress(b)        pairwise_ncd.py:78  (deflate level 6, +6 wrapper)     */
+    SNACC_BZIP2_9 = 3  /* bz2.compress(b)         pairwise_ncd.py:76  (bzip2 level 9, 900 kB blocks)    */
 };
 
 /* NCD formulas for snacc_ncd */
@@ -136,7 +137,11 @@ int snacc_last_kernel_ms(const snacc_ctx *ctx, double *ms, int64_t *launches);
  * "launches", "packed_jobs", "bytewise_jobs", "deflate_serial_jobs" (pair streams of a deflate call that took
  * the full serial parse after their canonical-stream shortcut met a block that might be stored),
  * "deflate_parallel_prep_seqs" (sequences whose parse alone was done in parallel chunks), "lz4_segments"
- * (segments per tile of the last linked-regime LZ4 pair launch) */
+ * (segments per tile of the last linked-regime LZ4 pair launch), "bzip2_blocks" (blocks sorted and counted),
+ * "bzip2_smem_blocks" (of those, sorted in shared memory), "bzip2_prefix_blocks" (closed blocks of an x taken from an
+ * earlier computation instead of being recomputed), "bzip2_rle_gather_ms", "bzip2_bwt_small_ms", "bzip2_bwt_large_ms",
+ * "bzip2_bits_ms" (device time of the bzip2 stages: RLE1 + block gather, BWT in shared / global memory, MTF + Huffman
+ * table choice + bit count) */
 int snacc_get_stat(const snacc_ctx *ctx, const char *name, double *out);
 /* tunables: 0 = default.  `streams_in_flight` bounds the number of concurrently parsed streams;
  * `invalidate_caches` (any value) drops every per-sequence precomputation so the next call redoes it;
@@ -144,7 +149,9 @@ int snacc_get_stat(const snacc_ctx *ctx, const char *name, double *out);
  * the full serial parse instead of the canonical symbol stream of y; `deflate_junction` 2 computes every junction
  * table without the 6-byte-index shortcut, `deflate_index6` 0 every match table from the 3-byte chain walk
  * `deflate_parallel_prep` 0 parses every sequence alone serially, `deflate_tail_index` 0 builds the whole 3-byte
- * index for x-only sequences, `lz4_segments` k forces k segments per LZ4 tile (all for tests: same results). */
+ * index for x-only sequences, `lz4_segments` k forces k segments per LZ4 tile, `bzip2_smem` 0 sorts every bzip2 block
+ * in global memory, `bzip2_prefix` 0 recomputes the closed blocks of x for every job x.y (all for tests: same
+ * results). */
 int snacc_set_option(snacc_ctx *ctx, const char *name, int64_t value);
 
 #ifdef __cplusplus

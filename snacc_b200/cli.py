@@ -117,7 +117,7 @@ def _parse_bool(ctx, param, value):
               type=click.Path(dir_okay=True, file_okay=False, resolve_path=True), default=None,
               help="Not supported on the GPU path (only sizes are produced).")
 @click.option("-c", "--compression", default="lzma", type=click.Choice(["lzma", "gzip", "bzip2", "zlib", "lz4"]),
-              help="The compression algorithm to use. The GPU path supports lz4, gzip and zlib.")
+              help="The compression algorithm to use. The GPU path supports lz4, gzip, zlib and bzip2.")
 @click.option("--show-progress/--no-show-progress", "showProgress", default=True,
               help="Accepted for compatibility.")
 @click.option("-r", "--reverse_complement", is_flag=True, default=False,
@@ -138,10 +138,11 @@ def cli(sequences, fasta, directories, numThreads, compression, showProgress, sa
     if saveCompression:
         raise click.UsageError("-s/--save-compression is not supported on the GPU path: compressed streams are "
                                "never materialised, only their sizes are computed")
-    if compression not in ("lz4", "gzip", "zlib"):
-        raise click.UsageError(f"-c {compression} is not supported on the GPU path (supported: lz4, gzip, zlib); "
-                               "there is no CPU fallback" + (" -- lzma is the reference's default (cli.py:52), so pass "
-                                                             "-c lz4, -c gzip or -c zlib explicitly"
+    if compression not in ("lz4", "gzip", "zlib", "bzip2"):
+        raise click.UsageError(f"-c {compression} is not supported on the GPU path (supported: lz4, gzip, zlib, "
+                               "bzip2); there is no CPU fallback" + (" -- lzma is the reference's default (cli.py:52), "
+                                                                     "so pass -c lz4, -c gzip, -c zlib or -c bzip2 "
+                                                                     "explicitly"
                                                              if compression == "lzma" else ""))
     if reverse_compliment is not None:
         reverse_complement = reverse_compliment

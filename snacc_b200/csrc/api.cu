@@ -21,6 +21,7 @@
 #include "lz4_packed.cuh"
 #include "deflate.cuh"
 #include "upgma.cuh"
+#include "bzip2.cuh"
 
 using namespace snacc;
 
@@ -71,7 +72,7 @@ struct snacc_ctx {
 
     // working memory
     uint8_t *d_work = nullptr; size_t work_bytes = 0;
-    void *d_scratch[14] = {nullptr}; size_t scratch_cap[14] = {0};   // per-call argument arrays, grown on demand, never
+    void *d_scratch[23] = {nullptr}; size_t scratch_cap[23] = {0};   // per-call argument arrays, grown on demand, never
                                                                    // freed between calls (all use is ordered on `stream`)
     unsigned long long *d_counter = nullptr;
     int32_t *d_jobx = nullptr, *d_joby = nullptr; int64_t job_cap = 0;
@@ -84,6 +85,18 @@ struct snacc_ctx {
     cudaEvent_t evm0 = nullptr, evm1 = nullptr;
 
     DeflateState dfl;
+
+    // bzip2 (bzip2.cuh): RLE1 of every sequence, its emission-start flags (a host copy plans the block cuts), where the
+    // open block of each sequence alone starts, and the bits of its closed blocks once computed
+    int bz_use_smem = 1, bz_use_prefix = 1;     // options "bzip2_smem", "bzip2_prefix" (0: for tests, same results)
+    bool bz_ready = false;
+    uint8_t *d_bz_rle = nullptr, *d_bz_flag = nullptr; BzSeq *d_bz_info = nullptr; uint64_t bz_rle_cap = 0;
+    unsigned long long *d_bz_seq_bits = nullptr;
+    std::vector<BzSeq> h_bz_info; std::vector<uint8_t> h_bz_flag, h_bz_pdone;
+    std::vector<uint32_t> h_bz_open, h_bz_nclosed;
+    int64_t bz_blocks = 0, bz_smem_blocks = 0, bz_prefix_blocks = 0;
+    double bz_ms[4] = {0, 0, 0, 0};            // RLE1 + gather, BWT small, BWT large, MTF + selection + bits
+    cudaEvent_t bz_ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
 };
 
 #define CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { \
@@ -327,6 +340,11 @@ static void free_corpus(snacc_ctx *ctx)
     ctx->corpus_dirty = 0;
     ctx->h_packable.clear(); ctx->h_ck_have.clear();
     ctx->n_seqs = 0; ctx->n_slots = 0;
+    cudaFree(ctx->d_bz_rle); ctx->d_bz_rle = nullptr;
+    cudaFree(ctx->d_bz_flag); ctx->d_bz_flag = nullptr;
+    cudaFree(ctx->d_bz_info); ctx->d_bz_info = nullptr;
+    cudaFree(ctx->d_bz_seq_bits); ctx->d_bz_seq_bits = nullptr;
+    ctx->bz_rle_cap = 0; ctx->bz_ready = false;
     deflate_free_corpus(ctx->dfl);
 }
 
@@ -344,6 +362,10 @@ extern "C" int snacc_ctx_create(int device_id, snacc_ctx **out)
         cudaEventCreate(&ctx->ev0) != cudaSuccess || cudaEventCreate(&ctx->ev1) != cudaSuccess ||
         cudaEventCreate(&ctx->evm0) != cudaSuccess || cudaEventCreate(&ctx->evm1) != cudaSuccess ||
         cudaMalloc(&ctx->d_counter, 64) != cudaSuccess) {
+        delete ctx;
+        return SNACC_ERR_CUDA;
+    }
+    for (cudaEvent_t &e : ctx->bz_ev) if (cudaEventCreate(&e) != cudaSuccess) {
         delete ctx;
         return SNACC_ERR_CUDA;
     }
@@ -367,6 +389,7 @@ extern "C" void snacc_ctx_destroy(snacc_ctx *ctx)
     cudaFree(ctx->d_jobx); cudaFree(ctx->d_joby); cudaFree(ctx->d_out);
     cudaEventDestroy(ctx->ev0); cudaEventDestroy(ctx->ev1);
     cudaEventDestroy(ctx->evm0); cudaEventDestroy(ctx->evm1);
+    for (cudaEvent_t e : ctx->bz_ev) cudaEventDestroy(e);
     cudaStreamDestroy(ctx->stream);
     delete ctx;
 }
@@ -515,6 +538,7 @@ static int upload_impl(snacc_ctx *ctx, const void *bytes, bool on_device, const 
     if (same_shape) {
         std::fill(ctx->ckpt_done.begin(), ctx->ckpt_done.end(), 0);
         deflate_invalidate(ctx->dfl);
+        ctx->bz_ready = false;
         ctx->n_seqs = 0;                                     // (restored below; a failure in between leaves no corpus)
     } else {
         free_corpus(ctx);
@@ -986,6 +1010,185 @@ static int run_lz4(snacc_ctx *ctx, const int32_t *h_x, const int32_t *h_y, int64
     return SNACC_OK;
 }
 
+// ---------------------------------------------------------------------------------------------
+// K5: bzip2 (bzip2.cuh).  RLE1 of every sequence once per upload; then per call the host cuts every job into blocks
+// (x's closed blocks once per x, the rest of each job from x's open tail, the junction and RLE1(y)) and the blocks go
+// through fixed-size batches: gather, BWT (shared memory up to BZ_SMEM_MAX_N bytes, else global scratch), MTF + table
+// choice + bit count.  Device memory of a batch is bounded by BZ_BATCH_BYTES whatever the number of jobs.
+// ---------------------------------------------------------------------------------------------
+constexpr uint64_t BZ_BATCH_BYTES = 192ull << 20;
+constexpr size_t BZ_BATCH_BLOCKS = 1 << 16;
+
+static int bz_prepare(snacc_ctx *ctx)
+{
+    NvtxRange nvtx_("snacc_b200: bzip2 RLE1");
+    const int32_t n = ctx->n_seqs;
+    ctx->h_bz_info.assign((size_t)n, BzSeq{});
+    uint64_t cap = 0;
+    for (int32_t i = 0; i < n; ++i) { ctx->h_bz_info[i].roff = cap; cap += (uint64_t)ctx->h_len[i] / 4 * 5 + 16; }
+    if (cap > ctx->bz_rle_cap) {
+        cudaFree(ctx->d_bz_rle); cudaFree(ctx->d_bz_flag); ctx->d_bz_rle = ctx->d_bz_flag = nullptr; ctx->bz_rle_cap = 0;
+        CK(cudaMalloc(&ctx->d_bz_rle, cap));
+        CK(cudaMalloc(&ctx->d_bz_flag, cap));
+        ctx->bz_rle_cap = cap;
+    }
+    if (!ctx->d_bz_info) CK(cudaMalloc(&ctx->d_bz_info, sizeof(BzSeq) * n));
+    if (!ctx->d_bz_seq_bits) CK(cudaMalloc(&ctx->d_bz_seq_bits, sizeof(unsigned long long) * n));
+    CK(cudaMemsetAsync(ctx->d_bz_seq_bits, 0, sizeof(unsigned long long) * n, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->d_bz_info, ctx->h_bz_info.data(), sizeof(BzSeq) * n, cudaMemcpyHostToDevice, ctx->stream));
+    std::vector<int32_t> all((size_t)n);
+    for (int32_t i = 0; i < n; ++i) all[i] = i;
+    int32_t *d_all = nullptr;
+    int rs = scratch(ctx, 14, sizeof(int32_t) * n, (void **)&d_all); if (rs) return rs;
+    CK(cudaMemcpyAsync(d_all, all.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice, ctx->stream));
+    bz_rle_kernel<<<(n + 31) / 32, 32, 0, ctx->stream>>>(ctx->d_corpus, ctx->d_off, ctx->d_len, d_all, n, ctx->d_bz_rle,
+                                                         ctx->d_bz_flag, ctx->d_bz_info);
+    CK(cudaGetLastError());
+    ctx->last_launches++;
+    ctx->h_bz_flag.resize(cap);
+    CK(cudaMemcpyAsync(ctx->h_bz_info.data(), ctx->d_bz_info, sizeof(BzSeq) * n, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->h_bz_flag.data(), ctx->d_bz_flag, cap, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    // where the last block of each sequence alone starts: the blocks before it close the same way in every x.y
+    ctx->h_bz_open.assign((size_t)n, 0); ctx->h_bz_nclosed.assign((size_t)n, 0); ctx->h_bz_pdone.assign((size_t)n, 0);
+    std::vector<BzWin> wins;
+    for (int32_t i = 0; i < n; ++i) {
+        const BzSeq &si = ctx->h_bz_info[i];
+        if (si.rlen <= BZ_NBLOCK_MAX) continue;
+        const uint8_t *f = ctx->h_bz_flag.data() + si.roff;
+        wins.clear();
+        bz_cut(bz_view_single(0, si.rlen), f, f, wins);
+        ctx->h_bz_open[i] = wins.back().v0;
+        ctx->h_bz_nclosed[i] = (uint32_t)wins.size() - 1;
+    }
+    ctx->bz_ready = true;
+    return SNACC_OK;
+}
+
+static int bz_run_batch(snacc_ctx *ctx, const BzBlock *blocks, size_t nb, uint64_t bytes,
+                        unsigned long long *d_job_bits)
+{
+    NvtxRange nvtx_("snacc_b200: bzip2 batch");
+    std::vector<int32_t> small, large;
+    for (size_t k = 0; k < nb; ++k)
+        ((ctx->bz_use_smem && blocks[k].n <= BZ_SMEM_MAX_N) ? small : large).push_back((int32_t)k);
+    BzBlock *d_blocks = nullptr; int32_t *d_small = nullptr, *d_large = nullptr;
+    uint8_t *d_buf = nullptr, *d_bwt = nullptr; uint16_t *d_mtf = nullptr; uint32_t *d_sort = nullptr;
+    int rs = scratch(ctx, 15, sizeof(BzBlock) * nb, (void **)&d_blocks); if (rs) return rs;
+    rs = scratch(ctx, 16, sizeof(int32_t) * (small.size() + 1), (void **)&d_small); if (rs) return rs;
+    rs = scratch(ctx, 17, sizeof(int32_t) * (large.size() + 1), (void **)&d_large); if (rs) return rs;
+    rs = scratch(ctx, 18, bytes, (void **)&d_buf); if (rs) return rs;
+    rs = scratch(ctx, 19, bytes, (void **)&d_bwt); if (rs) return rs;
+    rs = scratch(ctx, 20, sizeof(uint16_t) * (bytes + nb), (void **)&d_mtf); if (rs) return rs;
+    if (!large.empty()) {
+        // the global-memory sort's 4 arrays of 32-bit words per block byte
+        rs = ensure_work(ctx, 16 * bytes); if (rs) return rs;
+        d_sort = (uint32_t *)ctx->d_work;
+    }
+    CK(cudaMemcpyAsync(d_blocks, blocks, sizeof(BzBlock) * nb, cudaMemcpyHostToDevice, ctx->stream));
+    if (!small.empty()) CK(cudaMemcpyAsync(d_small, small.data(), sizeof(int32_t) * small.size(), cudaMemcpyHostToDevice, ctx->stream));
+    if (!large.empty()) CK(cudaMemcpyAsync(d_large, large.data(), sizeof(int32_t) * large.size(), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaEventRecord(ctx->bz_ev[0], ctx->stream));
+    bz_gather_kernel<<<(unsigned)nb, 256, 0, ctx->stream>>>(d_blocks, ctx->d_bz_info, ctx->d_bz_rle, ctx->d_bz_flag, d_buf);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ctx->bz_ev[1], ctx->stream));
+    if (!small.empty()) {
+        CK(cudaFuncSetAttribute(bz_bwt_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BZ_SMEM_BYTES));
+        bz_bwt_smem_kernel<<<(unsigned)small.size(), BZ_SORT_THREADS, BZ_SMEM_BYTES, ctx->stream>>>(d_blocks, d_small, d_buf, d_bwt);
+        CK(cudaGetLastError());
+    }
+    CK(cudaEventRecord(ctx->bz_ev[2], ctx->stream));
+    if (!large.empty()) {
+        bz_bwt_global_kernel<<<(unsigned)large.size(), BZ_SORT_THREADS, 0, ctx->stream>>>(d_blocks, d_large, d_buf, d_bwt, d_sort);
+        CK(cudaGetLastError());
+    }
+    CK(cudaEventRecord(ctx->bz_ev[3], ctx->stream));
+    CK(cudaFuncSetAttribute(bz_bits_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BZ_BITS_DYN_SMEM));
+    bz_bits_kernel<<<(unsigned)nb, BZ_BITS_THREADS, BZ_BITS_DYN_SMEM, ctx->stream>>>(d_blocks, d_bwt, d_mtf, d_job_bits,
+                                                                                    ctx->d_bz_seq_bits);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ctx->bz_ev[4], ctx->stream));
+    CK(cudaEventSynchronize(ctx->bz_ev[4]));
+    for (int s = 0; s < 4; ++s) {
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, ctx->bz_ev[s], ctx->bz_ev[s + 1]));
+        ctx->bz_ms[s] += ms;
+    }
+    ctx->last_launches += 2 + !small.empty() + !large.empty();
+    ctx->bz_blocks += (int64_t)nb;
+    ctx->bz_smem_blocks += (int64_t)small.size();
+    return SNACC_OK;
+}
+
+static int run_bzip2(snacc_ctx *ctx, const int32_t *xs, const int32_t *ys, int64_t n_jobs)
+{
+    ctx->bz_blocks = ctx->bz_smem_blocks = ctx->bz_prefix_blocks = 0;
+    for (double &m : ctx->bz_ms) m = 0;
+    if (!ctx->bz_ready) {
+        CK(cudaEventRecord(ctx->bz_ev[0], ctx->stream));
+        int r = bz_prepare(ctx);
+        if (r) return r;
+        CK(cudaEventRecord(ctx->bz_ev[1], ctx->stream));
+        CK(cudaEventSynchronize(ctx->bz_ev[1]));
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, ctx->bz_ev[0], ctx->bz_ev[1]));
+        ctx->bz_ms[0] += ms;
+    }
+    unsigned long long *d_job_bits = nullptr; uint8_t *d_use_prefix = nullptr;
+    int rs = scratch(ctx, 21, sizeof(unsigned long long) * n_jobs, (void **)&d_job_bits); if (rs) return rs;
+    rs = scratch(ctx, 22, (size_t)n_jobs, (void **)&d_use_prefix); if (rs) return rs;
+    CK(cudaMemsetAsync(d_job_bits, 0, sizeof(unsigned long long) * n_jobs, ctx->stream));
+    std::vector<uint8_t> use_prefix((size_t)n_jobs, 0);
+    std::vector<BzBlock> batch;
+    batch.reserve(BZ_BATCH_BLOCKS);
+    uint64_t bytes = 0;
+    std::vector<BzWin> wins;
+    const uint8_t *hf = ctx->h_bz_flag.data();
+    int64_t computed_closed = 0, used_closed = 0;
+    // blocks of the view v of job/sequence `dst` go into the batch, which runs whenever it is full
+    auto add = [&](int64_t dst, int32_t x, int32_t y, const BzView &v) -> int {
+        const BzSeq &sx = ctx->h_bz_info[x], &sy = ctx->h_bz_info[y < 0 ? x : y];
+        wins.clear();
+        bz_cut(v, hf + sx.roff, hf + sy.roff, wins);
+        for (const BzWin &w : wins) {
+            if (batch.size() == BZ_BATCH_BLOCKS || bytes + w.n > BZ_BATCH_BYTES) {
+                int r = bz_run_batch(ctx, batch.data(), batch.size(), bytes, d_job_bits);
+                if (r) return r;
+                batch.clear(); bytes = 0;
+            }
+            batch.push_back(BzBlock{dst, bytes, x, y, w.v0, w.n, v});
+            bytes += (w.n + 15) & ~15u;
+        }
+        return SNACC_OK;
+    };
+    for (int64_t k = 0; k < n_jobs; ++k) {
+        const int32_t x = xs[k], y = ys ? ys[k] : -1;
+        const uint32_t open = ctx->h_bz_open[x];
+        int r;
+        if (open) {
+            if (ctx->bz_use_prefix) {
+                use_prefix[k] = 1;
+                used_closed += ctx->h_bz_nclosed[x];
+                if (!ctx->h_bz_pdone[x]) {
+                    ctx->h_bz_pdone[x] = 1;
+                    computed_closed += ctx->h_bz_nclosed[x];
+                    if ((r = add(-1 - (int64_t)x, x, -1, bz_view_single(0, open)))) return r;
+                }
+            } else if ((r = add(k, x, -1, bz_view_single(0, open)))) return r;
+        }
+        const BzSeq &sx = ctx->h_bz_info[x];
+        if ((r = add(k, x, y, y < 0 ? bz_view_single(open, sx.rlen) : bz_view_pair(sx, open, ctx->h_bz_info[y])))) return r;
+    }
+    if (!batch.empty()) { int r = bz_run_batch(ctx, batch.data(), batch.size(), bytes, d_job_bits); if (r) return r; }
+    ctx->bz_prefix_blocks = used_closed - computed_closed;
+    CK(cudaMemcpyAsync(d_use_prefix, use_prefix.data(), (size_t)n_jobs, cudaMemcpyHostToDevice, ctx->stream));
+    const int blocks = (int)std::min<int64_t>((n_jobs + 255) / 256, 148 * 8);
+    bz_finish_kernel<<<blocks, 256, 0, ctx->stream>>>(d_job_bits, ctx->d_bz_seq_bits, ctx->d_jobx, d_use_prefix, n_jobs, ctx->d_out);
+    CK(cudaGetLastError());
+    ctx->last_launches++;
+    return SNACC_OK;
+}
+
 static int64_t wrapper_bytes(int codec) { return codec == SNACC_GZIP9 ? 18 : codec == SNACC_ZLIB6 ? 6 : 0; }
 
 // common driver: job lists on host -> sizes on host
@@ -995,8 +1198,8 @@ static int sizes_impl(snacc_ctx *ctx, int codec, const int32_t *xs, const int32_
     std::lock_guard<std::mutex> lock(ctx->mu);
     ctx->err.clear();
     if (!ctx->n_seqs) FAIL(SNACC_ERR_STATE, "nothing uploaded");
-    if (codec != SNACC_LZ4F && codec != SNACC_GZIP9 && codec != SNACC_ZLIB6)
-        FAIL(SNACC_ERR_CODEC, "codec not supported on the GPU path (supported: lz4, gzip, zlib)");
+    if (codec != SNACC_LZ4F && codec != SNACC_GZIP9 && codec != SNACC_ZLIB6 && codec != SNACC_BZIP2_9)
+        FAIL(SNACC_ERR_CODEC, "codec not supported on the GPU path (supported: lz4, gzip, zlib, bzip2)");
     if (n_jobs < 0 || (n_jobs && (!xs || !out))) FAIL(SNACC_ERR_ARG, "bad job list");
     if (n_jobs == 0) return SNACC_OK;
     for (int64_t k = 0; k < n_jobs; ++k) {
@@ -1013,6 +1216,7 @@ static int sizes_impl(snacc_ctx *ctx, int codec, const int32_t *xs, const int32_
     ctx->last_launches = 0;
     CK(cudaEventRecord(ctx->ev0, ctx->stream));
     if (codec == SNACC_LZ4F) r = run_lz4(ctx, xs, ys, n_jobs);
+    else if (codec == SNACC_BZIP2_9) r = run_bzip2(ctx, xs, ys, n_jobs);
     else {
         DeflateCorpus dc{ctx->d_corpus, ctx->d_off, ctx->d_len, ctx->h_off.data(), ctx->h_len.data(), ctx->n_seqs};
         r = deflate_run(ctx->dfl, dc, codec == SNACC_GZIP9 ? 9 : 6, xs, ys, ctx->d_jobx, ys ? ctx->d_joby : nullptr,
@@ -1025,7 +1229,8 @@ static int sizes_impl(snacc_ctx *ctx, int codec, const int32_t *xs, const int32_
     float ms = 0.f;
     CK(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
     ctx->last_ms = ms;
-    if (codec != SNACC_LZ4F) ctx->last_main_ms = ctx->dfl.main_ms;
+    if (codec == SNACC_GZIP9 || codec == SNACC_ZLIB6) ctx->last_main_ms = ctx->dfl.main_ms;
+    if (codec == SNACC_BZIP2_9) ctx->last_main_ms = ctx->bz_ms[1] + ctx->bz_ms[2];
     if (codec == SNACC_LZ4F) {
         CK(cudaEventElapsedTime(&ms, ctx->evm0, ctx->evm1)); ctx->last_main_ms = ms;
         // packed pair streams that could not use their checkpoint exactly (-1) are redone byte-wise
@@ -1241,6 +1446,13 @@ extern "C" int snacc_get_stat(const snacc_ctx *ctx, const char *name, double *ou
     if (!strcmp(name, "lz4_segments")) { *out = (double)ctx->last_pk_segments; return SNACC_OK; }
     if (!strcmp(name, "deflate_serial_jobs")) { *out = (double)ctx->dfl.serial_jobs; return SNACC_OK; }
     if (!strcmp(name, "deflate_parallel_prep_seqs")) { *out = (double)ctx->dfl.parallel_prep_seqs; return SNACC_OK; }
+    if (!strcmp(name, "bzip2_blocks")) { *out = (double)ctx->bz_blocks; return SNACC_OK; }
+    if (!strcmp(name, "bzip2_smem_blocks")) { *out = (double)ctx->bz_smem_blocks; return SNACC_OK; }
+    if (!strcmp(name, "bzip2_prefix_blocks")) { *out = (double)ctx->bz_prefix_blocks; return SNACC_OK; }
+    if (!strcmp(name, "bzip2_rle_gather_ms")) { *out = ctx->bz_ms[0]; return SNACC_OK; }
+    if (!strcmp(name, "bzip2_bwt_small_ms")) { *out = ctx->bz_ms[1]; return SNACC_OK; }
+    if (!strcmp(name, "bzip2_bwt_large_ms")) { *out = ctx->bz_ms[2]; return SNACC_OK; }
+    if (!strcmp(name, "bzip2_bits_ms")) { *out = ctx->bz_ms[3]; return SNACC_OK; }
     return SNACC_ERR_ARG;
 }
 
@@ -1256,12 +1468,15 @@ extern "C" int snacc_set_option(snacc_ctx *ctx, const char *name, int64_t value)
     if (!strcmp(name, "deflate_parallel_prep")) { ctx->dfl.use_parallel_prep = value ? 1 : 0; return SNACC_OK; }
     if (!strcmp(name, "deflate_tail_index")) { ctx->dfl.use_tail_index = value ? 1 : 0; return SNACC_OK; }
     if (!strcmp(name, "deflate_junction")) { ctx->dfl.junction_impl = value == 2 ? 2 : 3; return SNACC_OK; }
+    if (!strcmp(name, "bzip2_smem")) { ctx->bz_use_smem = value ? 1 : 0; return SNACC_OK; }
+    if (!strcmp(name, "bzip2_prefix")) { ctx->bz_use_prefix = value ? 1 : 0; ctx->bz_ready = false; return SNACC_OK; }
     if (!strcmp(name, "invalidate_caches")) {
         // forget every per-sequence precomputation (prefix checkpoints ...) so the next sizes call
         // redoes the whole job; used by bench.py so that no step reuses work of an earlier step
         std::fill(ctx->ckpt_done.begin(), ctx->ckpt_done.end(), 0);
         std::fill(ctx->h_ck_have.begin(), ctx->h_ck_have.end(), 0);
         deflate_invalidate(ctx->dfl);
+        ctx->bz_ready = false;
         return SNACC_OK;
     }
     ctx->err = std::string("unknown option: ") + name;

@@ -10,7 +10,7 @@ import numpy as np
 
 from . import _build
 
-CODEC_IDS = {"lz4": 0, "gzip": 1, "zlib": 2}
+CODEC_IDS = {"lz4": 0, "gzip": 1, "zlib": 2, "bzip2": 3}
 GETSIZEOF_BIAS = 33       # sys.getsizeof(b"") on 64-bit CPython 3 (reference pairwise_ncd.py:90)
 
 _STATUS = {-1: "CUDA error", -2: "bad argument", -3: "empty sequence", -4: "codec not supported on the GPU path",
@@ -234,5 +234,5 @@ class Engine:
 
 def _codec(algorithm):
     if algorithm not in CODEC_IDS:
-        raise KeyError(f"compression '{algorithm}' is not supported on the GPU path (supported: lz4, gzip, zlib)")
+        raise KeyError(f"compression '{algorithm}' is not supported on the GPU path (supported: lz4, gzip, zlib, bzip2)")
     return CODEC_IDS[algorithm]

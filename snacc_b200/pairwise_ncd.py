@@ -69,7 +69,7 @@ def compressed_size(sequences, algorithm, reverse_complement=False, save_directo
     ``sys.getsizeof``.  Routed through a batch of one on the GPU; thread-safe."""
     ext = _EXT[algorithm]            # KeyError for an unknown algorithm, like the reference
     if algorithm not in CODEC_IDS:
-        raise KeyError(f"compression '{algorithm}' is not supported on the GPU path (supported: lz4, gzip, zlib)")
+        raise KeyError(f"compression '{algorithm}' is not supported on the GPU path (supported: lz4, gzip, zlib, bzip2)")
     if save_directory:
         raise NotImplementedError("save_directory is not supported on the GPU path: only sizes are produced, "
                                   f"no {ext} stream is materialised")
@@ -105,7 +105,7 @@ def ncd_matrix(files, algorithm, reverse_complement=False, fast_mode=False, gpus
     ranks (``sharding.run_multi_gpu``) and returns rank 0's result; ``gpus`` in (None, 1) uses this process's GPU."""
     from . import sharding
     if algorithm not in CODEC_IDS:
-        raise KeyError(f"compression '{algorithm}' is not supported on the GPU path (supported: lz4, gzip, zlib)")
+        raise KeyError(f"compression '{algorithm}' is not supported on the GPU path (supported: lz4, gzip, zlib, bzip2)")
     files = [Path(f) for f in files]
     if gpus is not None and int(gpus) > 1 and sharding._dist() is None and engine is None:
         return sharding.run_multi_gpu(files, algorithm, reverse_complement, fast_mode, int(gpus))
