@@ -34,7 +34,8 @@ enum snacc_status {
     SNACC_ERR_EMPTY = -3,       /* a sequence is empty (reference raises ValueError, pairwise_ncd.py:37) */
     SNACC_ERR_CODEC = -4,       /* codec not supported on the GPU path (reference: KeyError / other libs) */
     SNACC_ERR_STATE = -5,       /* nothing uploaded yet */
-    SNACC_ERR_TOO_LARGE = -6    /* a stream would exceed 2 GiB - 1 */
+    SNACC_ERR_TOO_LARGE = -6    /* a stream would exceed 2 GiB - 1, or a deflate call cannot fit its x-side state,
+                                   working buffers and one y in device memory (message: bytes needed, bytes free) */
 };
 
 /* codec ids: which reference compressor call is reproduced */
@@ -136,7 +137,10 @@ int snacc_last_kernel_ms(const snacc_ctx *ctx, double *ms, int64_t *launches);
 /* named statistics of the last sizes call: "main_kernel_ms" (dominant kernel only), "total_kernel_ms",
  * "launches", "packed_jobs", "bytewise_jobs", "deflate_serial_jobs" (pair streams of a deflate call that took
  * the full serial parse after their canonical-stream shortcut met a block that might be stored),
- * "deflate_parallel_prep_seqs" (sequences whose parse alone was done in parallel chunks), "lz4_segments"
+ * "deflate_parallel_prep_seqs" (sequences whose parse alone was done in parallel chunks), "deflate_bands" (y layouts
+ * of the last deflate call: 1 when its state fit in device memory at once), "deflate_state_bytes" (peak device bytes of
+ * deflate per-sequence state plus working buffers during the last deflate call), "deflate_prepared_seqs" (full
+ * preparations -- index, match table, parse alone -- the last deflate call made), "lz4_segments"
  * (segments per tile of the last linked-regime LZ4 pair launch), "bzip2_blocks" (blocks sorted and counted),
  * "bzip2_smem_blocks" (of those, sorted in shared memory), "bzip2_prefix_blocks" (closed blocks of an x taken from an
  * earlier computation instead of being recomputed), "bzip2_rle_gather_ms", "bzip2_bwt_small_ms", "bzip2_bwt_large_ms",
@@ -149,7 +153,8 @@ int snacc_get_stat(const snacc_ctx *ctx, const char *name, double *out);
  * the full serial parse instead of the canonical symbol stream of y; `deflate_junction` 2 computes every junction
  * table without the 6-byte-index shortcut, `deflate_index6` 0 every match table from the 3-byte chain walk
  * `deflate_parallel_prep` 0 parses every sequence alone serially, `deflate_tail_index` 0 builds the whole 3-byte
- * index for x-only sequences, `lz4_segments` k forces k segments per LZ4 tile, `bzip2_smem` 0 sorts every bzip2 block
+ * index for x-only sequences, `deflate_band_bytes` b > 0 caps the deflate y-side state of one band at b bytes (0: plan
+ * from free device memory), `lz4_segments` k forces k segments per LZ4 tile, `bzip2_smem` 0 sorts every bzip2 block
  * in global memory, `bzip2_prefix` 0 recomputes the closed blocks of x for every job x.y (all for tests: same
  * results). */
 int snacc_set_option(snacc_ctx *ctx, const char *name, int64_t value);

@@ -1446,6 +1446,9 @@ extern "C" int snacc_get_stat(const snacc_ctx *ctx, const char *name, double *ou
     if (!strcmp(name, "lz4_segments")) { *out = (double)ctx->last_pk_segments; return SNACC_OK; }
     if (!strcmp(name, "deflate_serial_jobs")) { *out = (double)ctx->dfl.serial_jobs; return SNACC_OK; }
     if (!strcmp(name, "deflate_parallel_prep_seqs")) { *out = (double)ctx->dfl.parallel_prep_seqs; return SNACC_OK; }
+    if (!strcmp(name, "deflate_bands")) { *out = (double)ctx->dfl.bands; return SNACC_OK; }
+    if (!strcmp(name, "deflate_state_bytes")) { *out = (double)ctx->dfl.peak; return SNACC_OK; }
+    if (!strcmp(name, "deflate_prepared_seqs")) { *out = (double)ctx->dfl.prepared_seqs; return SNACC_OK; }
     if (!strcmp(name, "bzip2_blocks")) { *out = (double)ctx->bz_blocks; return SNACC_OK; }
     if (!strcmp(name, "bzip2_smem_blocks")) { *out = (double)ctx->bz_smem_blocks; return SNACC_OK; }
     if (!strcmp(name, "bzip2_prefix_blocks")) { *out = (double)ctx->bz_prefix_blocks; return SNACC_OK; }
@@ -1468,6 +1471,7 @@ extern "C" int snacc_set_option(snacc_ctx *ctx, const char *name, int64_t value)
     if (!strcmp(name, "deflate_parallel_prep")) { ctx->dfl.use_parallel_prep = value ? 1 : 0; return SNACC_OK; }
     if (!strcmp(name, "deflate_tail_index")) { ctx->dfl.use_tail_index = value ? 1 : 0; return SNACC_OK; }
     if (!strcmp(name, "deflate_junction")) { ctx->dfl.junction_impl = value == 2 ? 2 : 3; return SNACC_OK; }
+    if (!strcmp(name, "deflate_band_bytes")) { ctx->dfl.band_bytes = value < 0 ? 0 : value; return SNACC_OK; }
     if (!strcmp(name, "bzip2_smem")) { ctx->bz_use_smem = value ? 1 : 0; return SNACC_OK; }
     if (!strcmp(name, "bzip2_prefix")) { ctx->bz_use_prefix = value ? 1 : 0; ctx->bz_ready = false; return SNACC_OK; }
     if (!strcmp(name, "invalidate_caches")) {

@@ -40,8 +40,12 @@
 // candidate replaces the best only when strictly longer; the walk stops at nice_length; lengths are
 // capped by min(258, bytes left); a length-3 match farther than 4096 is dropped.
 #pragma once
+#include "../../include/snacc_b200.h"     // status codes (SNACC_ERR_TOO_LARGE)
 #include "common.cuh"
+#include <algorithm>
 #include <string>
+#include <unordered_map>
+#include <utility>
 #include <vector>
 
 namespace snacc {
@@ -1323,26 +1327,43 @@ static_assert(DFL_JSTRIDE % 8 == 0, "junction slices must start on 32-byte bound
 // ------------------------------------------------------------------------------------------------
 // kernels
 // ------------------------------------------------------------------------------------------------
+// A 3-byte index slice is one block: DFL_BROW words of bucket starts (DFL_HASH + 1 used), then the sorted positions.  It
+// lives in the y-side pool (the whole index of a sequence of the y layout) or in the x-side pool (its tail slice).
+constexpr uint32_t DFL_BROW = DFL_HASH + 8;
+
+// Device state is split by role.  x side (every sequence): record, tail index, tail packs.  y side (only the sequences
+// of the current y layout, DeflateState::ylist): whole index, F, head tables, canonical stream.  Per-sequence tables of
+// the y side are addressed through poff (per-position arrays) and yslot (fixed-size rows).
 struct DflCorpus {
     const uint8_t *corpus; const uint64_t *off; const uint32_t *len;   // padded byte corpus (api.cu)
-    const uint64_t *poff;        // per sequence: offset of its slice in `order` / F arrays
-    uint32_t *order;             // all sequences
-    uint32_t *bstart;            // per sequence DFL_HASH + 1 entries
-    // head of every sequence (its first DFL_JY positions), for the junction of the pair streams it ends:
-    uint16_t *head_order;        // per sequence DFL_JY entries: the indexed head positions sorted by (hash, position)
-    uint16_t *head_visit;        // per sequence and level DFL_JY entries: how longest_match went in the sequence alone
+    const uint64_t *poff;        // per y-side sequence: offset of its slice in the F / FQ arrays and the order6 window
+    uint32_t *const *ix;         // per sequence: its current 3-byte index slice (bucket starts, then positions)
+    const uint32_t *yslot;       // per y-side sequence: its row of head_order, head_visit and bstart6
+    // whole 3-byte index slices of the y side, the one of sequence sq at poff[sq] + yslot[sq] * DFL_BROW: a sequence is
+    // parsed alone only while it is in the y layout, and the kernels that do so address its index from here, as
+    // arithmetic the compiler may redo instead of keeping a loaded pointer live through the parse
+    uint32_t *yindex;
+    // head of every y-side sequence (its first DFL_JY positions), for the junction of the pair streams it ends:
+    uint16_t *head_order;        // per y slot DFL_JY entries: the indexed head positions sorted by (hash, position)
+    uint16_t *head_visit;        // per y slot and level DFL_JY entries: how longest_match went in the sequence alone
     // tail of every sequence, for the junction of the pair streams it starts:
     uint16_t *tail_cnt;          // per sequence DFL_HASH entries: bucket entries at or after dfl_tail3_from(len)
     uint16_t *tail6_order;       // per sequence DFL_T6 entries   } 6-byte index of the tail (DflTail6)
     uint16_t *tail6_start;       // per sequence DFL_H6 + 1 entries }
     // transient 6-byte index of whole sequences (DflIndex6): order6 is a window buffer addressed like `order`
     uint32_t *order6;
-    uint32_t *bstart6;           // per sequence DFL_HASH + 1 entries
+    uint32_t *bstart6;           // per y slot DFL_HASH + 1 entries
     // first position of the 3-byte index: 0, or len - DFL_XTAIL for a sequence that is only ever the x of pair streams
     // here (its record came from another rank): the junction walks reach at most 264 + 32 768 positions back from its end
     const uint32_t *ifrom;
 };
 constexpr uint32_t DFL_XTAIL = 40960;
+
+// (the table is rewritten by the host between launches only)
+__device__ __forceinline__ uint32_t *dfl_ix(const DflCorpus &c, int32_t s)
+{
+    return reinterpret_cast<uint32_t *>(__ldg(reinterpret_cast<const unsigned long long *>(c.ix + s)));
+}
 
 SNACC_HD Stream dfl_make_stream(const DflCorpus &c, int32_t x, int32_t y)
 {
@@ -1353,20 +1374,32 @@ SNACC_HD Stream dfl_make_stream(const DflCorpus &c, int32_t x, int32_t y)
     else        { s.y = s.x + s.lx;          s.n = s.lx; }
     return s;
 }
+// the pair stream x.y (y >= 0): each part's current index
 __device__ __forceinline__ DflStream dfl_make(const DflCorpus &c, int32_t x, int32_t y)
 {
     DflStream d;
     d.s = dfl_make_stream(c, x, y);
-    d.pair = y >= 0;
-    d.ix.order = c.order + c.poff[x]; d.ix.bstart = c.bstart + (size_t)x * (DFL_HASH + 1);
-    if (y >= 0) { d.iy.order = c.order + c.poff[y]; d.iy.bstart = c.bstart + (size_t)y * (DFL_HASH + 1); }
-    else d.iy = d.ix;
+    d.pair = true;
+    const uint32_t *ix = dfl_ix(c, x), *iy = dfl_ix(c, y);
+    d.ix.bstart = ix; d.ix.order = ix + DFL_BROW;
+    d.iy.bstart = iy; d.iy.order = iy + DFL_BROW;
+    return d;
+}
+// sequence sq alone: only parsed while it is in the y layout, so its index is the whole one there
+__device__ __forceinline__ DflStream dfl_make_alone(const DflCorpus &c, int32_t sq)
+{
+    DflStream d;
+    d.s = dfl_make_stream(c, sq, -1);
+    d.pair = false;
+    const uint32_t *ix = c.yindex + c.poff[sq] + (size_t)c.yslot[sq] * DFL_BROW;
+    d.ix.bstart = ix; d.ix.order = ix + DFL_BROW;
+    d.iy = d.ix;
     return d;
 }
 
 // K3a: index of a sequence = its positions sorted by (hash, position): a stable LSD radix sort on the 15-bit hash in
 // two passes (low 8 bits, high 7 bits).  The sort key is recomputed from the bytes, only positions move.
-//   KIND 0: the 3-byte chain hash over positions [0, len - 2) -> c.order / c.bstart;
+//   KIND 0: the 3-byte chain hash over positions [ifrom, len - 2) -> c.ix[sq];
 //   KIND 1: the 6-byte hash over positions [0, len - 5) -> c.order6 / c.bstart6 (DflIndex6).
 // A tile is 8192 consecutive keys handled by one CTA of 32 warps; warp w takes keys [256 w, 256 (w + 1)) of the tile in
 // 8 rounds of 32, so (warp, round, lane) order is key order and ranks come out stable: inside a round from
@@ -1389,6 +1422,7 @@ SNACC_HD uint32_t dfl_rx_tiles(uint32_t n) { return (n + DFL_RX_TILE - 1) / DFL_
 
 // SCATTER = false: digit totals of every tile -> hist[(seq slot * 256 + digit) * max_tiles + tile]
 // SCATTER = true : hist holds the exclusive scan of those totals; keys go to their sorted place
+// Scratch (src_all, and dst_all of pass 0) is addressed by poff; the 3-byte index lands in c.ix[sq], the 6-byte one in dst_all + poff.
 template <int KIND, int PASS, bool SCATTER>
 __global__ void __launch_bounds__(DFL_RX_THREADS)
 dfl_radix_kernel(DflCorpus c, const int32_t *__restrict__ seqs, uint32_t max_tiles, uint32_t *__restrict__ hist,
@@ -1402,7 +1436,7 @@ dfl_radix_kernel(DflCorpus c, const int32_t *__restrict__ seqs, uint32_t max_til
     if (tile * DFL_RX_TILE >= n) return;
     const uint8_t *p = c.corpus + c.off[sq];
     const uint32_t *src = src_all + c.poff[sq];
-    uint32_t *dst = dst_all + c.poff[sq];
+    uint32_t *dst = (KIND == 0 && PASS == 1) ? dfl_ix(c, sq) + DFL_BROW : dst_all + c.poff[sq];
     const uint32_t lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     for (uint32_t i = threadIdx.x; i < 32 * 256; i += blockDim.x) (&wcnt[0][0])[i] = 0;
     __syncthreads();
@@ -1465,8 +1499,8 @@ dfl_index_bounds_kernel(DflCorpus c, const int32_t *__restrict__ seqs)
     const int32_t sq = seqs[blockIdx.y];
     const uint32_t n = dfl_index_n<KIND>(c, sq);
     const uint8_t *p = c.corpus + c.off[sq];
-    const uint32_t *order = (KIND == 0 ? c.order : c.order6) + c.poff[sq];
-    uint32_t *bstart = (KIND == 0 ? c.bstart : c.bstart6) + (size_t)sq * (DFL_HASH + 1);
+    const uint32_t *order = KIND == 0 ? dfl_ix(c, sq) + DFL_BROW : c.order6 + c.poff[sq];
+    uint32_t *bstart = KIND == 0 ? dfl_ix(c, sq) : c.bstart6 + (size_t)c.yslot[sq] * (DFL_HASH + 1);
     for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
         const uint32_t h = dfl_index_hash<KIND>(p, order[k]);
         if (k == 0 || dfl_index_hash<KIND>(p, order[k - 1]) != h) bstart[h] = k;
@@ -1480,7 +1514,7 @@ dfl_index_fill_kernel(DflCorpus c, const int32_t *__restrict__ seqs, int phase)
     __shared__ uint32_t part[1024];
     const int32_t sq = seqs[blockIdx.x];
     const uint32_t n = dfl_index_n<KIND>(c, sq);
-    uint32_t *bstart = (KIND == 0 ? c.bstart : c.bstart6) + (size_t)sq * (DFL_HASH + 1);
+    uint32_t *bstart = KIND == 0 ? dfl_ix(c, sq) : c.bstart6 + (size_t)c.yslot[sq] * (DFL_HASH + 1);
     const uint32_t per = DFL_HASH / 1024;
     if (phase == 0) {
         for (uint32_t i = threadIdx.x; i < DFL_HASH; i += blockDim.x) bstart[i] = 0xffffffffu;
@@ -1514,25 +1548,27 @@ dfl_match_kernel(DflCorpus c, const int32_t *__restrict__ seqs, int32_t n_seqs, 
     const DflConfig cfg = dfl_config(level);
     for (int32_t t = blockIdx.y; t < n_seqs; t += gridDim.y) {
         const int32_t sq = seqs[t];
-        const DflStream d = dfl_make(c, sq, -1);
+        const DflStream d = dfl_make_alone(c, sq);
         const uint32_t len = d.s.n;
         const uint32_t nidx = len >= 3 ? len - 2 : 0;
         uint32_t *f = F + c.poff[sq];
         uint32_t *fq = FQ ? FQ + c.poff[sq] : nullptr;
-        const DflIndex6 i6{c.order6 ? c.order6 + c.poff[sq] : nullptr, c.bstart6 + (size_t)sq * (DFL_HASH + 1)};
+        const DflIndex6 i6{c.order6 ? c.order6 + c.poff[sq] : nullptr, c.bstart6 + (size_t)c.yslot[sq] * (DFL_HASH + 1)};
+        uint16_t *hvis = c.head_visit + (size_t)c.yslot[sq] * DFL_JY;
         for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < len; k += gridDim.x * blockDim.x) {
             if (k >= nidx) { f[k] = 0; if (fq) fq[k] = 0; continue; }       // the last two positions: no string, no search
             const uint32_t p = d.ix.order[k];
             uint32_t q, visit;
             f[p] = dfl_match_word(d, p, cfg, k, c.order6 ? &i6 : nullptr, &q, &visit);
             if (fq) fq[p] = q;
-            if (p < DFL_JY) c.head_visit[(size_t)sq * DFL_JY + p] = (uint16_t)visit;
+            if (p < DFL_JY) hvis[p] = (uint16_t)visit;
         }
     }
 }
 
 // K3b': head order of the listed sequences: the first min(len - 2, DFL_JY) positions sorted by (hash, position),
-// taken bucket by bucket from the full index (a bucket's head positions are a prefix of it).  One CTA per sequence.
+// taken bucket by bucket from the full index (a bucket's head positions are a prefix of it), and the tail counts of the
+// x side.  head_order == nullptr: x-side index, tail counts only.  One CTA per sequence.
 __global__ void __launch_bounds__(1024)
 dfl_head_kernel(DflCorpus c, const int32_t *__restrict__ seqs, int32_t n_seqs)
 {
@@ -1540,9 +1576,7 @@ dfl_head_kernel(DflCorpus c, const int32_t *__restrict__ seqs, int32_t n_seqs)
     __shared__ uint32_t wsum[32];
     for (int32_t t = blockIdx.x; t < n_seqs; t += gridDim.x) {
         const int32_t sq = seqs[t];
-        const uint32_t *order = c.order + c.poff[sq];
-        const uint32_t *bstart = c.bstart + (size_t)sq * (DFL_HASH + 1);
-        uint16_t *ho = c.head_order + (size_t)sq * DFL_JY;
+        const uint32_t *bstart = dfl_ix(c, sq), *order = bstart + DFL_BROW;
         __syncthreads();
         const uint32_t tail_from = dfl_tail3_from(c.len[sq]);
         uint16_t *tc = c.tail_cnt + (size_t)sq * DFL_HASH;
@@ -1551,7 +1585,8 @@ dfl_head_kernel(DflCorpus c, const int32_t *__restrict__ seqs, int32_t n_seqs)
             hcnt[h] = lo < hi ? dfl_lower_bound(order, lo, hi, DFL_JY) - lo : 0;
             tc[h] = (uint16_t)(lo < hi ? hi - dfl_lower_bound(order, lo, hi, tail_from) : 0);
         }
-        if (c.ifrom[sq]) continue;                           // tail-only index (x role): no head order
+        if (c.ifrom[sq] || !c.head_order) continue;          // x-side index: no head order
+        uint16_t *ho = c.head_order + (size_t)c.yslot[sq] * DFL_JY;
         __syncthreads();
         // exclusive scan over DFL_HASH counters: 32 per thread
         const uint32_t per = DFL_HASH / 1024;
@@ -1642,7 +1677,7 @@ dfl_junction_kernel(DflCorpus c, const DflPair *__restrict__ pairs, int32_t n_pa
         uint32_t *fq = FJQ ? FJQ + (size_t)b * DFL_JSTRIDE : nullptr;
         const uint32_t *fy = F + c.poff[y];
         const uint32_t *fqy = FQ ? FQ + c.poff[y] : nullptr;
-        const uint16_t *ho = c.head_order + (size_t)y * DFL_JY, *hv = c.head_visit + (size_t)y * DFL_JY;
+        const uint16_t *ho = c.head_order + (size_t)c.yslot[y] * DFL_JY, *hv = c.head_visit + (size_t)c.yslot[y] * DFL_JY;
         const uint32_t u_end = jxl + jyl;
         const bool by_hash = impl != 3 || level != 9;
         const int32_t xi = pairs[b].x;
@@ -1771,7 +1806,7 @@ dfl_prep_kernel(DflCorpus c, const int32_t *__restrict__ seqs, int32_t n_seqs, i
     const uint32_t tid = threadIdx.x, C = DFL_PREP_CHUNK;
     for (int32_t t = blockIdx.x; t < n_seqs; t += gridDim.x) {
         const int32_t sq = seqs[t];
-        const DflStream d = dfl_make(c, sq, -1);
+        const DflStream d = dfl_make_alone(c, sq);
         const uint32_t n = d.s.n, n_pad = (n + 7) & ~7u, jx0 = dfl_jx0(n);
         const uint32_t *fsrc = F + c.poff[sq];
         DflFView fv;
@@ -1836,7 +1871,7 @@ dfl_chunk_scan_kernel(DflCorpus c, DflChunkArgs a, int level, const uint32_t *__
     const DflConfig cfg = dfl_config(level);
     for (int32_t i = blockIdx.y; i < a.n_seqs; i += gridDim.y) {
         const int32_t sq = a.seqs[i];
-        const DflStream d = dfl_make(c, sq, -1);
+        const DflStream d = dfl_make_alone(c, sq);
         const uint32_t n = d.s.n, K = dfl_chunk_count(n), E = dfl_chunk_end(n);
         const uint32_t *f = F + c.poff[sq], *q = FQ ? FQ + c.poff[sq] : nullptr;
         for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < K; k += gridDim.x * blockDim.x) {
@@ -1864,7 +1899,7 @@ dfl_chunk_pass_kernel(DflCorpus c, DflChunkArgs a, int level, const uint32_t *__
     for (int32_t i = blockIdx.y; i < a.n_seqs; i += gridDim.y) {
         if (MODE == 2 && a.fail[i]) continue;
         const int32_t sq = a.seqs[i];
-        const DflStream d = dfl_make(c, sq, -1);
+        const DflStream d = dfl_make_alone(c, sq);
         const uint32_t n = d.s.n, K = dfl_chunk_count(n), E = dfl_chunk_end(n);
         const uint32_t *f = F + c.poff[sq], *q = FQ ? FQ + c.poff[sq] : nullptr;
         for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < K; k += gridDim.x * blockDim.x) {
@@ -1929,7 +1964,7 @@ dfl_alone_kernel(DflCorpus c, DflChunkArgs a, int level, const uint32_t *__restr
         for (uint32_t k = threadIdx.x; k < DFL_D_CODES; k += blockDim.x) sm.df[k] = 0;
         __syncthreads();
         if (threadIdx.x) continue;
-        const DflStream d = dfl_make(c, sq, -1);
+        const DflStream d = dfl_make_alone(c, sq);
         const uint32_t n = d.s.n, jx0 = dfl_jx0(n);
         DflFView fv;
         fv.fx = fv.fy = fv.fj = F + c.poff[sq]; fv.jx0 = fv.jend = fv.lx = n;
@@ -2013,75 +2048,157 @@ struct DeflateCorpus {
     const uint64_t *h_off; const uint32_t *h_len; int32_t n_seqs;
 };
 
+// Device state of the deflate codecs, split by the role a sequence plays (DflCorpus):
+//   x side, every sequence: its record (checkpoint + size alone), its tail 3-byte index (the whole index with
+//     deflate_tail_index 0), tail counts and tail 6-byte pack -- what a pair stream x.* needs of x;
+//   y side, only the sequences of `ylist` (the current y layout): whole index, F (+ FQ), head order and visits, 6-byte
+//     index starts and the canonical symbol stream -- what a pair stream *.y needs of y, and what the parse of a
+//     sequence alone needs to produce its record.
+// deflate_run plans the y layouts of a call from free device memory: everything in one layout when it fits (the state
+// then stays resident for later calls), else bands of y sequences, each prepared, used and dropped in turn.
 struct DeflateState {
-    // per-corpus
-    uint64_t *d_poff = nullptr; std::vector<uint64_t> h_poff; uint64_t total = 0;
-    uint32_t *d_order = nullptr, *d_bstart = nullptr;
-    uint16_t *d_head_order = nullptr, *d_head_visit[2] = {nullptr, nullptr};
+    int32_t n_seqs = 0;
+    // ---- x side ----
+    int x_whole = 0;                               // the x index pool holds whole indexes (made with deflate_tail_index 0)
+    std::vector<uint64_t> h_xoff; uint64_t x_total = 0;
+    uint64_t *d_xoff = nullptr;                    // per sequence: offset of its positions in the x sort scratch window
+    uint32_t *d_xindex = nullptr;                  // x index slices: sequence i at h_xoff[i] + i * DFL_BROW
     uint16_t *d_tail_cnt = nullptr, *d_tail6_order = nullptr, *d_tail6_start = nullptr;
     uint32_t *d_ifrom = nullptr; std::vector<uint32_t> h_ifrom;     // first position of every 3-byte index (DflCorpus::ifrom)
-    uint32_t *d_rx_hist = nullptr; size_t rx_cap = 0;   // radix-sort digit totals (dfl_build_index)
-    uint32_t *d_bstart6 = nullptr, *d_order6 = nullptr; uint64_t order6_cap = 0;   // 6-byte index: starts per sequence, window buffer
-    int use_index6 = 1;                            // 0: dfl_match_kernel always walks the 3-byte chain (tests)
-    int use_parallel_prep = 1;                     // 0: every sequence alone is parsed by the serial kernel (tests, A/B)
-    int use_tail_index = 1;                        // 0: x-role sequences get the whole 3-byte index too (tests, A/B)
-    int64_t parallel_prep_seqs = 0;                // sequences the chunked path finished in the last call
-    std::vector<uint8_t> indexed;                  // per sequence
+    uint32_t *d_cap = nullptr;                     // canonical stream capacity of every sequence (symbols)
+    uint32_t **d_ix = nullptr; std::vector<uint32_t *> h_ix;       // where each sequence's 3-byte index is (DflCorpus::ix)
+    std::vector<uint8_t> xindexed;                 // x index slice built
+    std::vector<uint8_t> have_ckpt[2];             // x-side record present (own parse or imported from another rank)
+    DflCkpt *d_ckpt[2] = {nullptr, nullptr};
+    int64_t *d_seq_size[2] = {nullptr, nullptr};
+    uint32_t *d_nsym[2] = {nullptr, nullptr};
+    // per-sequence addressing of the y side (x-side allocations, rewritten with every layout)
+    uint64_t *d_poff = nullptr, *d_soff = nullptr, *d_roff = nullptr; uint32_t *d_yslot = nullptr;
+    // ---- y side ----
+    std::vector<int32_t> ylist;
+    std::vector<uint32_t> h_yslot; std::vector<uint64_t> h_poff;
+    uint64_t y_total = 0, sym_total = 0, row_total = 0;
+    uint32_t *d_yindex = nullptr, *d_bstart6 = nullptr;     // y index slices: sequence i at h_poff[i] + h_yslot[i] * DFL_BROW
+    uint16_t *d_head_order = nullptr, *d_head_visit[2] = {nullptr, nullptr};
     uint32_t *d_F[2] = {nullptr, nullptr};         // level 9, level 6
     uint32_t *d_FQ = nullptr;                      // level 6 only: quartered-chain table
-    std::vector<uint8_t> have_F[2], have_prep[2];
-    std::vector<uint8_t> have_ckpt[2];             // x-side product present (own parse or imported from another rank): the
-                                                   // checkpoint a pair stream x.* resumes from and the size of x alone
-    DflCkpt *d_ckpt[2] = {nullptr, nullptr};
-    // canonical symbol streams (per level): pools + per-sequence geometry (shared by both levels)
-    uint64_t *d_soff = nullptr, *d_roff = nullptr; uint32_t *d_cap = nullptr;
-    uint64_t sym_total = 0, row_total = 0;
     uint32_t *d_sym_end[2] = {nullptr, nullptr}; uint16_t *d_sym_code[2] = {nullptr, nullptr};
-    uint32_t *d_cum[2] = {nullptr, nullptr}; uint32_t *d_nsym[2] = {nullptr, nullptr};
-    int64_t *d_seq_size[2] = {nullptr, nullptr};
-    int32_t n_seqs = 0;
-    // working memory
-    DflTrees *d_scratch2[2] = {nullptr, nullptr}; size_t scratch_n = 0;
-    uint32_t *d_FJ2[2] = {nullptr, nullptr}, *d_FJQ2[2] = {nullptr, nullptr}; size_t fj_pairs = 0;
+    uint32_t *d_cum[2] = {nullptr, nullptr};
+    std::vector<uint8_t> yindexed, have_F[2], have_prep[2];
+    // ---- working memory ----
+    uint32_t *d_rx_hist = nullptr; size_t rx_cap = 0;   // radix-sort digit totals (dfl_build_index)
+    uint32_t *d_order6 = nullptr; uint64_t order6_cap = 0;   // 6-byte index window
+    uint32_t *d_xtmp = nullptr; uint64_t xtmp_cap = 0;       // sort scratch of x index builds
+    DflTrees *d_scratch2[2] = {nullptr, nullptr}; size_t scratch_n[2] = {0, 0};
+    uint32_t *d_FJ2[2] = {nullptr, nullptr}, *d_FJQ2[2] = {nullptr, nullptr}; size_t fj_pairs[2] = {0, 0};
     DflPair *d_pairs2[2] = {nullptr, nullptr}; DflJob *d_jobs2[2] = {nullptr, nullptr};
     cudaStream_t stream2 = nullptr; cudaEvent_t ev_j[2] = {nullptr, nullptr}, ev_p[2] = {nullptr, nullptr};
     cudaEvent_t ev_t[2] = {nullptr, nullptr};      // timing of the junction kernel
     unsigned long long *d_counter2 = nullptr;
-    double main_ms = 0.0;
+    // ---- device bytes held, by kind: 0 x side, 1 y side, 2 preparation scratch (released at the end of every call),
+    //      3 pair-batch buffers (junction tables, parse scratch, job lists; kept for the next call of the same shape) ----
+    std::unordered_map<void *, std::pair<size_t, int>> held;
+    size_t live[4] = {0, 0, 0, 0}, peak = 0;
+    // ---- switches and statistics ----
+    int use_index6 = 1;                            // 0: dfl_match_kernel always walks the 3-byte chain (tests)
+    int use_parallel_prep = 1;                     // 0: every sequence alone is parsed by the serial kernel (tests, A/B)
+    int use_tail_index = 1;                        // 0: x-role sequences get the whole 3-byte index too (tests, A/B)
     int use_canon = 1;                             // 0: every pair stream takes the full serial parse (tests)
     int junction_impl = 3;                         // 2: no 6-byte-index shortcut in the junction walk (tests)
+    int64_t band_bytes = 0;                        // > 0: cap of the y layout of a band (tests); 0: plan from free memory
+    int64_t parallel_prep_seqs = 0;                // sequences the chunked path finished in the last call
     int64_t serial_jobs = 0;                       // pair jobs of the last call that fell back to it
+    int64_t bands = 0;                             // y layouts the last call went through
+    int64_t prepared_seqs = 0;                     // full preparations (index, F, parse alone) the last call made
+    double main_ms = 0.0;
 };
 
+template <typename T> static cudaError_t dfl_malloc(DeflateState &st, int kind, T **p, size_t bytes)
+{
+    *p = nullptr;
+    const cudaError_t e = cudaMalloc(p, bytes);
+    if (e != cudaSuccess) return e;
+    st.held[(void *)*p] = {bytes, kind};
+    st.live[kind] += bytes;
+    st.peak = std::max(st.peak, st.live[0] + st.live[1] + st.live[2] + st.live[3]);
+    return e;
+}
+template <typename T> static void dfl_free(DeflateState &st, T *&p)
+{
+    if (!p) return;
+    auto it = st.held.find((void *)p);
+    if (it != st.held.end()) { st.live[it->second.second] -= it->second.first; st.held.erase(it); }
+    cudaFree(p);
+    p = nullptr;
+}
+
+// ---- bytes per sequence of each side (what the planner counts; the allocations below follow the same sums) ----
+static inline uint64_t dfl_pad8(uint32_t len) { return ((uint64_t)len + 7) & ~7ull; }
+// canonical stream: room for one symbol per 4 bytes (DNA needs one per ~9); a sequence that needs more simply has no
+// canonical stream and its pair jobs take the serial parse
+static inline uint32_t dfl_canon_cap(uint32_t len) { return (len / 4 + 1024 + DFL_CUM_G - 1) / DFL_CUM_G * DFL_CUM_G; }
+static inline uint32_t dfl_xtail_from(uint32_t len) { return len > DFL_XTAIL ? len - DFL_XTAIL : 0u; }
+static inline uint64_t dfl_xslot(uint32_t len, int whole) { return whole ? dfl_pad8(len) : std::min<uint64_t>(dfl_pad8(len), DFL_XTAIL); }
+static inline uint64_t dfl_xbytes_fixed()
+{
+    return 4ull * DFL_BROW + 2ull * DFL_HASH + 2ull * DFL_T6 + 2ull * (DFL_H6 + 1)       // bstart, tail counts, tail pack
+         + 8 + 4 + 4 + 8 + 8 + 8 + 8 + 4;                                     // xoff ifrom cap ix poff soff roff yslot
+}
+static inline uint64_t dfl_xbytes_level() { return sizeof(DflCkpt) + 8 + 4; }
+static inline uint64_t dfl_ybytes(uint32_t len, int level)
+{
+    const uint64_t cap = dfl_canon_cap(len);
+    return dfl_pad8(len) * 4 * (level == 9 ? 2 : 3)                                 // order, F (, FQ)
+         + cap * 6 + (cap / DFL_CUM_G + 1) * DFL_CUM_W * 4                          // symbol ends + codes, cumulative rows
+         + 4ull * (DFL_BROW + DFL_HASH + 1) + 4ull * DFL_JY                         // bucket starts (3-, 6-byte), head order + visits
+         + (uint64_t)dfl_chunk_count(len) * (2 * DFL_CHUNK_WORDS + 3) * 4;          // chunk scratch of the parallel parse
+}
+
+static inline void deflate_drop_y(DeflateState &st)
+{
+    dfl_free(st, st.d_yindex); dfl_free(st, st.d_bstart6); dfl_free(st, st.d_head_order);
+    dfl_free(st, st.d_FQ);
+    for (int l = 0; l < 2; ++l) {
+        dfl_free(st, st.d_F[l]); dfl_free(st, st.d_head_visit[l]);
+        dfl_free(st, st.d_sym_end[l]); dfl_free(st, st.d_sym_code[l]); dfl_free(st, st.d_cum[l]);
+        std::fill(st.have_F[l].begin(), st.have_F[l].end(), 0);
+        std::fill(st.have_prep[l].begin(), st.have_prep[l].end(), 0);
+    }
+    for (int32_t i : st.ylist) { st.h_yslot[i] = DFL_NONE; st.yindexed[i] = 0; }
+    st.ylist.clear();
+    st.y_total = st.sym_total = st.row_total = 0;
+}
 static inline void deflate_free_corpus(DeflateState &st)
 {
-    cudaFree(st.d_poff); cudaFree(st.d_order); cudaFree(st.d_bstart);
-    cudaFree(st.d_FQ); st.d_FQ = nullptr;
-    cudaFree(st.d_soff); cudaFree(st.d_roff); cudaFree(st.d_cap);
-    cudaFree(st.d_head_order); st.d_head_order = nullptr;
-    cudaFree(st.d_tail_cnt); cudaFree(st.d_tail6_order); cudaFree(st.d_tail6_start); cudaFree(st.d_ifrom);
-    st.d_tail_cnt = st.d_tail6_order = st.d_tail6_start = nullptr; st.d_ifrom = nullptr; st.h_ifrom.clear();
-    cudaFree(st.d_bstart6); cudaFree(st.d_order6); st.d_bstart6 = st.d_order6 = nullptr; st.order6_cap = 0;
-    cudaFree(st.d_rx_hist); st.d_rx_hist = nullptr; st.rx_cap = 0;
-    for (int l = 0; l < 2; ++l) { cudaFree(st.d_head_visit[l]); st.d_head_visit[l] = nullptr; }
-    st.d_soff = st.d_roff = nullptr; st.d_cap = nullptr;
+    deflate_drop_y(st);
+    dfl_free(st, st.d_xoff); dfl_free(st, st.d_xindex);
+    dfl_free(st, st.d_tail_cnt); dfl_free(st, st.d_tail6_order); dfl_free(st, st.d_tail6_start);
+    dfl_free(st, st.d_ifrom); dfl_free(st, st.d_cap); dfl_free(st, st.d_ix);
+    dfl_free(st, st.d_poff); dfl_free(st, st.d_soff); dfl_free(st, st.d_roff); dfl_free(st, st.d_yslot);
+    dfl_free(st, st.d_bstart6); dfl_free(st, st.d_order6); st.order6_cap = 0;
+    dfl_free(st, st.d_rx_hist); st.rx_cap = 0;
+    dfl_free(st, st.d_xtmp); st.xtmp_cap = 0;
     for (int l = 0; l < 2; ++l) {
-        cudaFree(st.d_F[l]); cudaFree(st.d_ckpt[l]); st.d_F[l] = nullptr; st.d_ckpt[l] = nullptr;
-        cudaFree(st.d_sym_end[l]); cudaFree(st.d_sym_code[l]); cudaFree(st.d_cum[l]); cudaFree(st.d_nsym[l]);
-        cudaFree(st.d_seq_size[l]);
-        st.d_sym_end[l] = nullptr; st.d_sym_code[l] = nullptr; st.d_cum[l] = nullptr; st.d_nsym[l] = nullptr;
-        st.d_seq_size[l] = nullptr;
+        dfl_free(st, st.d_ckpt[l]); dfl_free(st, st.d_seq_size[l]); dfl_free(st, st.d_nsym[l]);
         st.have_F[l].clear(); st.have_prep[l].clear(); st.have_ckpt[l].clear();
     }
-    st.d_poff = nullptr; st.d_order = nullptr; st.d_bstart = nullptr; st.indexed.clear(); st.h_poff.clear();
-    st.n_seqs = 0; st.total = 0;
+    st.h_xoff.clear(); st.h_ifrom.clear(); st.h_ix.clear(); st.xindexed.clear();
+    st.h_yslot.clear(); st.h_poff.clear(); st.yindexed.clear();
+    st.n_seqs = 0; st.x_total = 0;
+}
+// the pair-batch buffers (junction tables, parse scratch, job lists)
+static inline void deflate_free_batches(DeflateState &st)
+{
+    for (int k = 0; k < 2; ++k) {
+        dfl_free(st, st.d_scratch2[k]); dfl_free(st, st.d_FJ2[k]); dfl_free(st, st.d_FJQ2[k]);
+        dfl_free(st, st.d_pairs2[k]); dfl_free(st, st.d_jobs2[k]);
+        st.scratch_n[k] = st.fj_pairs[k] = 0;
+    }
 }
 static inline void deflate_free_work(DeflateState &st)
 {
-    st.scratch_n = 0; st.fj_pairs = 0;
+    deflate_free_batches(st);
     for (int k = 0; k < 2; ++k) {
-        cudaFree(st.d_scratch2[k]); cudaFree(st.d_FJ2[k]); cudaFree(st.d_FJQ2[k]); cudaFree(st.d_pairs2[k]); cudaFree(st.d_jobs2[k]);
-        st.d_scratch2[k] = nullptr; st.d_FJ2[k] = st.d_FJQ2[k] = nullptr; st.d_pairs2[k] = nullptr; st.d_jobs2[k] = nullptr;
         if (st.ev_j[k]) cudaEventDestroy(st.ev_j[k]);
         if (st.ev_p[k]) cudaEventDestroy(st.ev_p[k]);
         if (st.ev_t[k]) cudaEventDestroy(st.ev_t[k]);
@@ -2089,11 +2206,12 @@ static inline void deflate_free_work(DeflateState &st)
     }
     if (st.stream2) cudaStreamDestroy(st.stream2);
     st.stream2 = nullptr;
-    cudaFree(st.d_counter2); st.d_counter2 = nullptr;
+    dfl_free(st, st.d_counter2);
 }
 static inline void deflate_invalidate(DeflateState &st)
 {
-    std::fill(st.indexed.begin(), st.indexed.end(), 0);
+    std::fill(st.xindexed.begin(), st.xindexed.end(), 0);
+    std::fill(st.yindexed.begin(), st.yindexed.end(), 0);
     for (int l = 0; l < 2; ++l) {
         std::fill(st.have_F[l].begin(), st.have_F[l].end(), 0);
         std::fill(st.have_prep[l].begin(), st.have_prep[l].end(), 0);
@@ -2118,9 +2236,11 @@ constexpr int DFL_PARSE_BLOCKS = 148 * 5;           // parse threads a batch is 
 constexpr size_t DFL_BATCH = (size_t)DFL_PARSE_BLOCKS * 64;   // pair streams per junction batch: one per parse thread (6.3 GB of
                                                     // junction F per buffer, two buffers; the parse is latency-bound, so
                                                     // its throughput is the number of streams in flight)
+constexpr uint64_t DFL_ORDER6_CAP = 192ull << 20;   // entries of the 6-byte index window: 768 MB at most
+constexpr int DFL_INDEX_GROUP = 64;                 // sequences per index build
 
 // build the KIND index of the listed sequences (radix sort, bucket starts); tmp: one scratch entry per position,
-// addressed like `order` (the F slices are used)
+// addressed like the F slices (c.poff)
 template <int KIND>
 static int dfl_build_index(DeflateState &st, const DflCorpus &c, const std::vector<int32_t> &list, const uint32_t *h_len,
                            uint32_t *tmp, cudaStream_t stream, int64_t *launches, std::string &err)
@@ -2134,14 +2254,14 @@ static int dfl_build_index(DeflateState &st, const DflCorpus &c, const std::vect
     const uint32_t max_tiles = std::max(1u, dfl_rx_tiles(mx));
     const size_t need = list.size() * 256 * (size_t)max_tiles;
     if (st.rx_cap < need) {
-        cudaFree(st.d_rx_hist); st.d_rx_hist = nullptr;
-        DCK(cudaMalloc(&st.d_rx_hist, sizeof(uint32_t) * need));
+        dfl_free(st, st.d_rx_hist); st.rx_cap = 0;
+        DCK(dfl_malloc(st, 2, &st.d_rx_hist, sizeof(uint32_t) * need));
         st.rx_cap = need;
     }
     int32_t *d_list = nullptr;
     if (dfl_upload(err, stream, list, &d_list)) return -1;
     const dim3 grid(max_tiles, (unsigned)list.size());
-    uint32_t *order = KIND == 0 ? c.order : c.order6;
+    uint32_t *order = KIND == 0 ? nullptr : c.order6;                  // (KIND 0: the slices of c.ix)
     DCK(cudaMemsetAsync(st.d_rx_hist, 0, sizeof(uint32_t) * need, stream));
     dfl_radix_kernel<KIND, 0, false><<<grid, DFL_RX_THREADS, 0, stream>>>(c, d_list, max_tiles, st.d_rx_hist, tmp, tmp);
     dfl_radix_scan_kernel<<<(unsigned)list.size(), 1024, 0, stream>>>(max_tiles, st.d_rx_hist);
@@ -2160,62 +2280,341 @@ static int dfl_build_index(DeflateState &st, const DflCorpus &c, const std::vect
     return 0;
 }
 
-// sizes of the raw deflate streams of the jobs (x alone when ys == nullptr) into d_out[0..n_jobs)
-// per-corpus and per-level device state (allocated on first use)
-static int deflate_ensure_alloc(DeflateState &st, const DeflateCorpus &dc, int level, cudaStream_t stream, std::string &err)
+// x side of every sequence (allocated on first use, and again when the x index layout changes)
+static int deflate_ensure_x(DeflateState &st, const DeflateCorpus &dc, int level, cudaStream_t stream, std::string &err)
 {
     const int li = level == 9 ? 0 : 1;
     const int32_t ns = dc.n_seqs;
-    if (st.n_seqs != ns || !st.d_poff) {
+    const int whole = st.use_tail_index ? 0 : 1;
+    if (st.n_seqs != ns || !st.d_xoff) {
         deflate_free_corpus(st);
         st.n_seqs = ns;
-        st.h_poff.assign(ns, 0);
-        std::vector<uint64_t> soff(ns), roff(ns);
         std::vector<uint32_t> cap(ns);
-        uint64_t t = 0, sy = 0, ro = 0;
-        for (int32_t i = 0; i < ns; ++i) {
-            st.h_poff[i] = t; t += ((uint64_t)dc.h_len[i] + 7) & ~7ull;
-            // canonical stream: room for one symbol per 4 bytes (DNA needs one per ~9); a sequence that needs more
-            // simply has no canonical stream and its pair jobs take the serial parse
-            cap[i] = (dc.h_len[i] / 4 + 1024 + DFL_CUM_G - 1) / DFL_CUM_G * DFL_CUM_G;
-            soff[i] = sy; sy += cap[i];
-            roff[i] = ro; ro += cap[i] / DFL_CUM_G + 1;
-        }
-        st.total = t; st.sym_total = sy; st.row_total = ro;
-        DCK(cudaMalloc(&st.d_poff, sizeof(uint64_t) * ns));
-        DCK(cudaMemcpyAsync(st.d_poff, st.h_poff.data(), sizeof(uint64_t) * ns, cudaMemcpyHostToDevice, stream));
-        DCK(cudaMalloc(&st.d_soff, sizeof(uint64_t) * ns));
-        DCK(cudaMalloc(&st.d_roff, sizeof(uint64_t) * ns));
-        DCK(cudaMalloc(&st.d_cap, sizeof(uint32_t) * ns));
-        DCK(cudaMemcpyAsync(st.d_soff, soff.data(), sizeof(uint64_t) * ns, cudaMemcpyHostToDevice, stream));
-        DCK(cudaMemcpyAsync(st.d_roff, roff.data(), sizeof(uint64_t) * ns, cudaMemcpyHostToDevice, stream));
+        for (int32_t i = 0; i < ns; ++i) cap[i] = dfl_canon_cap(dc.h_len[i]);
+        DCK(dfl_malloc(st, 0, &st.d_xoff, sizeof(uint64_t) * ns));
+        DCK(dfl_malloc(st, 0, &st.d_tail_cnt, sizeof(uint16_t) * (size_t)ns * DFL_HASH));
+        DCK(dfl_malloc(st, 0, &st.d_tail6_order, sizeof(uint16_t) * (size_t)ns * DFL_T6));
+        DCK(dfl_malloc(st, 0, &st.d_tail6_start, sizeof(uint16_t) * (size_t)ns * (DFL_H6 + 1)));
+        DCK(dfl_malloc(st, 0, &st.d_ifrom, sizeof(uint32_t) * ns));
+        DCK(dfl_malloc(st, 0, &st.d_cap, sizeof(uint32_t) * ns));
+        DCK(dfl_malloc(st, 0, &st.d_ix, sizeof(uint32_t *) * ns));
+        DCK(dfl_malloc(st, 0, &st.d_poff, sizeof(uint64_t) * ns));
+        DCK(dfl_malloc(st, 0, &st.d_soff, sizeof(uint64_t) * ns));
+        DCK(dfl_malloc(st, 0, &st.d_roff, sizeof(uint64_t) * ns));
+        DCK(dfl_malloc(st, 0, &st.d_yslot, sizeof(uint32_t) * ns));
         DCK(cudaMemcpyAsync(st.d_cap, cap.data(), sizeof(uint32_t) * ns, cudaMemcpyHostToDevice, stream));
+        DCK(cudaMemsetAsync(st.d_ifrom, 0, sizeof(uint32_t) * ns, stream));
         DCK(cudaStreamSynchronize(stream));
-        DCK(cudaMalloc(&st.d_order, sizeof(uint32_t) * (t + 16)));
-        DCK(cudaMalloc(&st.d_bstart, sizeof(uint32_t) * (size_t)ns * (DFL_HASH + 1)));
-        DCK(cudaMalloc(&st.d_head_order, sizeof(uint16_t) * (size_t)ns * DFL_JY));
-        DCK(cudaMalloc(&st.d_tail_cnt, sizeof(uint16_t) * (size_t)ns * DFL_HASH));
-        DCK(cudaMalloc(&st.d_bstart6, sizeof(uint32_t) * (size_t)ns * (DFL_HASH + 1)));
-        DCK(cudaMalloc(&st.d_tail6_order, sizeof(uint16_t) * (size_t)ns * DFL_T6));
-        DCK(cudaMalloc(&st.d_tail6_start, sizeof(uint16_t) * (size_t)ns * (DFL_H6 + 1)));
-        DCK(cudaMalloc(&st.d_ifrom, sizeof(uint32_t) * (size_t)ns));
-        DCK(cudaMemsetAsync(st.d_ifrom, 0, sizeof(uint32_t) * (size_t)ns, stream));
-        st.h_ifrom.assign(ns, 0);
-        st.indexed.assign(ns, 0);
+        st.h_ifrom.assign(ns, 0); st.h_ix.assign(ns, nullptr); st.xindexed.assign(ns, 0);
+        st.h_yslot.assign(ns, DFL_NONE); st.h_poff.assign(ns, 0); st.yindexed.assign(ns, 0);
         for (int l = 0; l < 2; ++l) { st.have_F[l].assign(ns, 0); st.have_prep[l].assign(ns, 0); st.have_ckpt[l].assign(ns, 0); }
+        st.x_whole = -1;
     }
-    if (!st.d_F[li]) {
-        DCK(cudaMalloc(&st.d_F[li], sizeof(uint32_t) * (st.total + 16)));
-        DCK(cudaMalloc(&st.d_ckpt[li], sizeof(DflCkpt) * ns));
-        DCK(cudaMalloc(&st.d_head_visit[li], sizeof(uint16_t) * (size_t)ns * DFL_JY));
-        if (level != 9) DCK(cudaMalloc(&st.d_FQ, sizeof(uint32_t) * (st.total + 16)));
-        DCK(cudaMalloc(&st.d_sym_end[li], sizeof(uint32_t) * (st.sym_total + 16)));
-        DCK(cudaMalloc(&st.d_sym_code[li], sizeof(uint16_t) * (st.sym_total + 16)));
-        DCK(cudaMalloc(&st.d_cum[li], sizeof(uint32_t) * st.row_total * DFL_CUM_W));
-        DCK(cudaMalloc(&st.d_nsym[li], sizeof(uint32_t) * ns));
-        DCK(cudaMalloc(&st.d_seq_size[li], sizeof(int64_t) * ns));
+    if (st.x_whole != whole) {
+        dfl_free(st, st.d_xindex);
+        std::fill(st.xindexed.begin(), st.xindexed.end(), 0);
+        st.h_xoff.assign(ns, 0);
+        uint64_t t = 0;
+        for (int32_t i = 0; i < ns; ++i) { st.h_xoff[i] = t; t += dfl_xslot(dc.h_len[i], whole); }
+        st.x_total = t;
+        DCK(dfl_malloc(st, 0, &st.d_xindex, sizeof(uint32_t) * (t + (uint64_t)ns * DFL_BROW + 16)));
+        DCK(cudaMemcpyAsync(st.d_xoff, st.h_xoff.data(), sizeof(uint64_t) * ns, cudaMemcpyHostToDevice, stream));
+        DCK(cudaStreamSynchronize(stream));
+        st.x_whole = whole;
+    }
+    if (!st.d_ckpt[li]) {
+        DCK(dfl_malloc(st, 0, &st.d_ckpt[li], sizeof(DflCkpt) * ns));
+        DCK(dfl_malloc(st, 0, &st.d_seq_size[li], sizeof(int64_t) * ns));
+        DCK(dfl_malloc(st, 0, &st.d_nsym[li], sizeof(uint32_t) * ns));
         DCK(cudaMemsetAsync(st.d_nsym[li], 0, sizeof(uint32_t) * ns, stream));
     }
+    return 0;
+}
+
+// the per-level arrays of the current y layout
+static int deflate_alloc_y_level(DeflateState &st, int level, std::string &err)
+{
+    const int li = level == 9 ? 0 : 1;
+    if (st.ylist.empty() || st.d_F[li]) return 0;
+    const size_t ny = st.ylist.size();
+    DCK(dfl_malloc(st, 1, &st.d_F[li], sizeof(uint32_t) * (st.y_total + 16)));
+    if (level != 9 && !st.d_FQ) DCK(dfl_malloc(st, 1, &st.d_FQ, sizeof(uint32_t) * (st.y_total + 16)));
+    DCK(dfl_malloc(st, 1, &st.d_head_visit[li], sizeof(uint16_t) * ny * DFL_JY));
+    DCK(dfl_malloc(st, 1, &st.d_sym_end[li], sizeof(uint32_t) * (st.sym_total + 16)));
+    DCK(dfl_malloc(st, 1, &st.d_sym_code[li], sizeof(uint16_t) * (st.sym_total + 16)));
+    DCK(dfl_malloc(st, 1, &st.d_cum[li], sizeof(uint32_t) * st.row_total * DFL_CUM_W));
+    return 0;
+}
+// (a failed allocation -- the device is shared -- leaves no layout rather than a layout with missing arrays)
+static int deflate_ensure_y_level(DeflateState &st, int level, std::string &err)
+{
+    if (deflate_alloc_y_level(st, level, err)) { deflate_drop_y(st); return -1; }
+    return 0;
+}
+
+static int deflate_layout_arrays(DeflateState &st, const DeflateCorpus &dc, int level, const std::vector<int32_t> &list,
+                                 cudaStream_t stream, std::string &err)
+{
+    deflate_drop_y(st);
+    const int32_t ns = dc.n_seqs;
+    std::vector<uint64_t> soff(ns, 0), roff(ns, 0);
+    uint64_t t = 0, sy = 0, ro = 0;
+    for (size_t k = 0; k < list.size(); ++k) {
+        const int32_t i = list[k];
+        const uint32_t cap = dfl_canon_cap(dc.h_len[i]);
+        st.h_yslot[i] = (uint32_t)k;
+        st.h_poff[i] = t; t += dfl_pad8(dc.h_len[i]);
+        soff[i] = sy; sy += cap;
+        roff[i] = ro; ro += cap / DFL_CUM_G + 1;
+    }
+    st.ylist = list;
+    st.y_total = t; st.sym_total = sy; st.row_total = ro;
+    DCK(cudaMemcpyAsync(st.d_poff, st.h_poff.data(), sizeof(uint64_t) * ns, cudaMemcpyHostToDevice, stream));
+    DCK(cudaMemcpyAsync(st.d_soff, soff.data(), sizeof(uint64_t) * ns, cudaMemcpyHostToDevice, stream));
+    DCK(cudaMemcpyAsync(st.d_roff, roff.data(), sizeof(uint64_t) * ns, cudaMemcpyHostToDevice, stream));
+    DCK(cudaMemcpyAsync(st.d_yslot, st.h_yslot.data(), sizeof(uint32_t) * ns, cudaMemcpyHostToDevice, stream));
+    DCK(cudaStreamSynchronize(stream));
+    const size_t ny = list.size();
+    DCK(dfl_malloc(st, 1, &st.d_yindex, sizeof(uint32_t) * (t + ny * DFL_BROW + 16)));
+    DCK(dfl_malloc(st, 1, &st.d_bstart6, sizeof(uint32_t) * ny * (DFL_HASH + 1)));
+    DCK(dfl_malloc(st, 1, &st.d_head_order, sizeof(uint16_t) * ny * DFL_JY));
+    return deflate_alloc_y_level(st, level, err);
+}
+// a new y layout holding exactly `list` (ascending): the previous one is dropped; on failure there is no layout
+static int deflate_set_layout(DeflateState &st, const DeflateCorpus &dc, int level, const std::vector<int32_t> &list,
+                              cudaStream_t stream, std::string &err)
+{
+    if (deflate_layout_arrays(st, dc, level, list, stream, err)) { deflate_drop_y(st); return -1; }
+    return 0;
+}
+
+// every sequence's 3-byte index: the whole one while it is in the y layout and built, else its x slice
+static int deflate_upload_ix(DeflateState &st, cudaStream_t stream, std::string &err)
+{
+    for (int32_t i = 0; i < st.n_seqs; ++i)
+        st.h_ix[i] = st.yindexed[i] ? st.d_yindex + st.h_poff[i] + (size_t)st.h_yslot[i] * DFL_BROW
+                                    : st.d_xindex + st.h_xoff[i] + (size_t)i * DFL_BROW;
+    DCK(cudaMemcpyAsync(st.d_ix, st.h_ix.data(), sizeof(uint32_t *) * st.n_seqs, cudaMemcpyHostToDevice, stream));
+    DCK(cudaStreamSynchronize(stream));
+    return 0;
+}
+
+static DflCorpus deflate_corpus(const DeflateState &st, const DeflateCorpus &dc, int li)
+{
+    return DflCorpus{dc.d_corpus, dc.d_off, dc.d_len, st.d_poff, st.d_ix, st.d_yslot, st.d_yindex,
+                     st.d_head_order, st.d_head_visit[li],
+                     st.d_tail_cnt, st.d_tail6_order, st.d_tail6_start, nullptr, st.d_bstart6, st.d_ifrom};
+}
+
+// the head order / tail counts and tail packs of sequences whose 3-byte index was just built
+static int dfl_index_packs(const DflCorpus &c, const std::vector<int32_t> &list, cudaStream_t stream, int64_t *launches,
+                           std::string &err)
+{
+    int32_t *d_list = nullptr;
+    if (dfl_upload(err, stream, list, &d_list)) return -1;
+    DCK(cudaFuncSetAttribute(dfl_head_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(DFL_HASH * 4)));
+    dfl_head_kernel<<<(unsigned)std::min<size_t>(list.size(), 148), 1024, DFL_HASH * 4, stream>>>(c, d_list, (int32_t)list.size());
+    DCK(cudaGetLastError());
+    const int t6_smem = (int)(DFL_H6 * 4 + DFL_T6 * 2);
+    DCK(cudaFuncSetAttribute(dfl_tail6_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, t6_smem));
+    dfl_tail6_kernel<<<(unsigned)std::min<size_t>(list.size(), 148 * 2), 32, t6_smem, stream>>>(c, d_list, (int32_t)list.size());
+    DCK(cudaGetLastError());
+    *launches += 3;
+    DCK(cudaStreamSynchronize(stream));
+    cudaFree(d_list);
+    return 0;
+}
+
+// x index slices of the listed sequences (their last DFL_XTAIL positions, or whole with deflate_tail_index 0): the
+// junction walks of a pair stream x.y reach at most 264 + 32 768 positions back from the end of x
+static int deflate_build_x(DeflateState &st, const DeflateCorpus &dc, int li, const std::vector<int32_t> &list,
+                           cudaStream_t stream, int64_t *launches, std::string &err)
+{
+    if (list.empty()) return 0;
+    NvtxRange nvtx_("snacc_b200: deflate x index (radix sort, tail packs)");
+    // window: the slices of up to DFL_INDEX_GROUP x-tail sequences, at least one whole slice (deflate_tail_index 0)
+    uint64_t sum = 0, big = 0;
+    for (int32_t i : list) { const uint64_t n = dfl_xslot(dc.h_len[i], st.x_whole); sum += n; big = std::max(big, n); }
+    const uint64_t cap = std::max(big, std::min<uint64_t>(sum, (uint64_t)DFL_INDEX_GROUP * DFL_XTAIL));
+    if (st.xtmp_cap < cap) { dfl_free(st, st.d_xtmp); st.xtmp_cap = 0; DCK(dfl_malloc(st, 2, &st.d_xtmp, sizeof(uint32_t) * (cap + 16))); st.xtmp_cap = cap; }
+    for (int32_t i : list) { st.h_ifrom[i] = st.x_whole ? 0u : dfl_xtail_from(dc.h_len[i]); st.xindexed[i] = 1; }
+    if (deflate_upload_ix(st, stream, err)) return -1;
+    DCK(cudaMemcpyAsync(st.d_ifrom, st.h_ifrom.data(), sizeof(uint32_t) * st.n_seqs, cudaMemcpyHostToDevice, stream));
+    DflCorpus c = deflate_corpus(st, dc, li);
+    for (int32_t i : list) if (st.yindexed[i]) { err = "deflate_build_x: sequence holds its whole index"; return -1; }
+    c.poff = st.d_xoff;                                                // sort scratch: a window addressed like the x slices
+    c.head_order = nullptr;                                            // tail counts only
+    size_t a = 0;
+    while (a < list.size()) {
+        size_t b = a + 1;
+        const uint64_t first = st.h_xoff[list[a]];
+        while (b < list.size() && b - a < (size_t)DFL_INDEX_GROUP &&
+               st.h_xoff[list[b]] + dfl_xslot(dc.h_len[list[b]], st.x_whole) - first <= st.xtmp_cap) ++b;
+        std::vector<int32_t> part(list.begin() + a, list.begin() + b);
+        if (dfl_build_index<0>(st, c, part, dc.h_len, st.d_xtmp - first, stream, launches, err)) return -1;
+        a = b;
+    }
+    return dfl_index_packs(c, list, stream, launches, err);
+}
+
+// the full preparation of the listed sequences of the y layout that lack it: whole index, F of this level and the
+// parse of the sequence alone (size, checkpoint, canonical symbol stream)
+static int deflate_prepare_y(DeflateState &st, const DeflateCorpus &dc, int level, const std::vector<int32_t> &list,
+                             cudaStream_t stream, int64_t *launches, std::string &err)
+{
+    const int li = level == 9 ? 0 : 1;
+    std::vector<int32_t> need_idx, need_f, need_prep;
+    for (int32_t i : list) {
+        if (!st.yindexed[i]) { need_idx.push_back(i); st.have_F[0][i] = st.have_F[1][i] = 0; }
+        if (!st.have_F[li][i] || !st.yindexed[i]) { need_f.push_back(i); st.have_prep[li][i] = 0; }
+        if (!st.have_prep[li][i]) need_prep.push_back(i);
+    }
+    if (need_prep.empty()) return 0;
+    st.prepared_seqs += (int64_t)need_prep.size();
+    uint32_t *FQ = level != 9 ? st.d_FQ : nullptr;
+    if (!need_idx.empty()) {
+        NvtxRange nvtx_("snacc_b200: deflate index (radix sort, head/tail packs)");
+        for (int32_t i : need_idx) { st.yindexed[i] = 1; st.h_ifrom[i] = 0; }
+        if (deflate_upload_ix(st, stream, err)) return -1;
+        DCK(cudaMemcpyAsync(st.d_ifrom, st.h_ifrom.data(), sizeof(uint32_t) * st.n_seqs, cudaMemcpyHostToDevice, stream));
+        const DflCorpus c = deflate_corpus(st, dc, li);
+        // the F slices of this level double as sort scratch; they are recomputed right below
+        for (size_t a0 = 0; a0 < need_idx.size(); a0 += DFL_INDEX_GROUP) {
+            std::vector<int32_t> part(need_idx.begin() + a0, need_idx.begin() + std::min(need_idx.size(), a0 + DFL_INDEX_GROUP));
+            if (dfl_build_index<0>(st, c, part, dc.h_len, st.d_F[li], stream, launches, err)) return -1;
+        }
+        if (dfl_index_packs(c, need_idx, stream, launches, err)) return -1;
+    }
+    const DflCorpus c = deflate_corpus(st, dc, li);
+    if (!need_f.empty()) {
+        NvtxRange nvtx_("snacc_b200: deflate match tables");
+        // level 9: runs of sequences whose index slices fit the window buffer get a transient 6-byte index first
+        // (dfl_match_word); level 6 always walks the chain (its limit of 128 binds everywhere on DNA)
+        const bool i6 = st.use_index6 && level == 9;
+        const uint64_t cap = std::min<uint64_t>(DFL_ORDER6_CAP, st.y_total);
+        if (i6 && st.order6_cap < cap) {
+            dfl_free(st, st.d_order6); st.order6_cap = 0;
+            DCK(dfl_malloc(st, 2, &st.d_order6, sizeof(uint32_t) * (cap + 16))); st.order6_cap = cap;
+        }
+        size_t a = 0;
+        while (a < need_f.size()) {
+            size_t b = a + 1;
+            const uint64_t first = st.h_poff[need_f[a]];
+            auto end_of = [&](int32_t i) { return st.h_poff[i] + dfl_pad8(dc.h_len[i]); };
+            while (b < need_f.size() && b - a < 64 && (!i6 || end_of(need_f[b]) - first <= st.order6_cap)) ++b;
+            const bool fits = i6 && end_of(need_f[b - 1]) - first <= st.order6_cap;   // (a single sequence longer than the buffer: no index)
+            std::vector<int32_t> part(need_f.begin() + a, need_f.begin() + b);
+            int32_t *d_list = nullptr;
+            if (dfl_upload(err, stream, part, &d_list)) return -1;
+            DflCorpus cm = c;
+            if (fits) {
+                cm.order6 = st.d_order6 - first;                               // addressed like F: + poff[sq]
+                if (dfl_build_index<1>(st, cm, part, dc.h_len, st.d_F[li], stream, launches, err)) return -1;
+            }
+            uint32_t mx = 0;
+            for (int32_t i : part) mx = std::max(mx, dc.h_len[i]);
+            dim3 grid(std::max(1u, std::min((mx + 255) / 256, 4096u)), (unsigned)part.size());
+            dfl_match_kernel<<<grid, 256, 0, stream>>>(cm, d_list, (int32_t)part.size(), level, st.d_F[li], FQ);
+            DCK(cudaGetLastError());
+            ++*launches;
+            DCK(cudaStreamSynchronize(stream));
+            cudaFree(d_list);
+            for (int32_t i : part) st.have_F[li][i] = 1;
+            a = b;
+        }
+    }
+    DflCanonPool cp{st.d_sym_end[li], st.d_sym_code[li], st.d_cum[li], st.d_soff, st.d_cap, st.d_roff, st.d_nsym[li],
+                    st.d_seq_size[li]};
+    NvtxRange nvtx_("snacc_b200: deflate sequence parses (sizes, checkpoints, canonical streams)");
+    // long sequences: chunks in parallel (dfl_chunk_*_kernel), then cumulative rows, then dfl_alone_kernel; the
+    // others -- and whatever the parallel path gives up on -- take the serial kernel
+    std::vector<int32_t> par, ser;
+    for (int32_t i : need_prep) (st.use_parallel_prep && dc.h_len[i] >= DFL_PAR_MIN ? par : ser).push_back(i);
+    auto run_serial = [&](const std::vector<int32_t> &list) -> int {
+        if (list.empty()) return 0;
+        int32_t *d_list = nullptr;
+        if (dfl_upload(err, stream, list, &d_list)) return -1;
+        DCK(cudaFuncSetAttribute(dfl_prep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DflPrepSmem)));
+        dfl_prep_kernel<<<(unsigned)std::min<size_t>(list.size(), 148 * 5), DFL_PREP_THREADS, sizeof(DflPrepSmem), stream>>>(
+            c, d_list, (int32_t)list.size(), level, st.d_F[li], FQ, st.d_ckpt[li], cp);
+        DCK(cudaGetLastError());
+        ++*launches;
+        DCK(cudaStreamSynchronize(stream));
+        cudaFree(d_list);
+        return 0;
+    };
+    auto run_cum = [&](const std::vector<int32_t> &list) -> int {
+        if (list.empty()) return 0;
+        int32_t *d_list = nullptr;
+        if (dfl_upload(err, stream, list, &d_list)) return -1;
+        uint32_t max_rows = 1;
+        for (int32_t i : list) max_rows = std::max(max_rows, dc.h_len[i] / 4 / DFL_CUM_G + 8);
+        dim3 grid(std::min(max_rows, 2048u), (unsigned)std::min<size_t>(list.size(), 64));
+        dfl_cum_chunk_kernel<<<grid, 64, 0, stream>>>(cp, d_list, (int32_t)list.size());
+        dfl_cum_scan_kernel<<<(unsigned)std::min<size_t>(list.size(), 148 * 4), DFL_CUM_W, 0, stream>>>(
+            cp, d_list, (int32_t)list.size());
+        DCK(cudaGetLastError());
+        *launches += 2;
+        DCK(cudaStreamSynchronize(stream));
+        cudaFree(d_list);
+        return 0;
+    };
+    if (!par.empty()) {
+        // per-chunk scratch of the listed sequences (2 x 128 B of bitmaps + 12 B per 8 KiB chunk)
+        std::vector<uint64_t> coff(par.size() + 1, 0);
+        uint32_t max_k = 1;
+        for (size_t k = 0; k < par.size(); ++k) {
+            const uint32_t K = dfl_chunk_count(dc.h_len[par[k]]);
+            coff[k + 1] = coff[k] + K; max_k = std::max(max_k, K);
+        }
+        const uint64_t tot = coff.back();
+        int32_t *d_list = nullptr; uint64_t *d_coff = nullptr; uint32_t *d_w = nullptr; int32_t *d_fail = nullptr;
+        if (dfl_upload(err, stream, par, &d_list)) return -1;
+        auto free_all = [&]() { cudaFree(d_list); cudaFree(d_coff); dfl_free(st, d_w); cudaFree(d_fail); };
+        if (cudaMalloc(&d_coff, sizeof(uint64_t) * coff.size()) != cudaSuccess ||
+            dfl_malloc(st, 2, &d_w, sizeof(uint32_t) * tot * (2 * DFL_CHUNK_WORDS + 3)) != cudaSuccess ||
+            cudaMalloc(&d_fail, sizeof(int32_t) * par.size()) != cudaSuccess) { free_all(); err = "cudaMalloc (chunk scratch) failed"; return -1; }
+        cudaMemcpyAsync(d_coff, coff.data(), sizeof(uint64_t) * coff.size(), cudaMemcpyHostToDevice, stream);
+        cudaMemsetAsync(d_fail, 0, sizeof(int32_t) * par.size(), stream);
+        DflChunkArgs a{d_list, d_coff, (int32_t)par.size(), d_w, d_w + tot * DFL_CHUNK_WORDS, d_w + tot * 2 * DFL_CHUNK_WORDS,
+                       d_w + tot * (2 * DFL_CHUNK_WORDS + 1), d_w + tot * (2 * DFL_CHUNK_WORDS + 2), d_fail};
+        dim3 grid((max_k + 127) / 128, (unsigned)std::min<size_t>(par.size(), 65535));
+        dfl_chunk_scan_kernel<<<grid, 128, 0, stream>>>(c, a, level, st.d_F[li], FQ);
+        dfl_chunk_pass_kernel<1><<<grid, 128, 0, stream>>>(c, a, level, st.d_F[li], FQ, cp);
+        dfl_chunk_offsets_kernel<<<(unsigned)((par.size() + 63) / 64), 64, 0, stream>>>(c, a, cp);
+        dfl_chunk_pass_kernel<2><<<grid, 128, 0, stream>>>(c, a, level, st.d_F[li], FQ, cp);
+        *launches += 4;
+        std::vector<int32_t> fail(par.size(), 0);
+        if (cudaGetLastError() != cudaSuccess ||
+            cudaMemcpyAsync(fail.data(), d_fail, sizeof(int32_t) * par.size(), cudaMemcpyDeviceToHost, stream) != cudaSuccess ||
+            cudaStreamSynchronize(stream) != cudaSuccess) { free_all(); err = "deflate chunk kernels failed"; return -1; }
+        std::vector<int32_t> ok;
+        for (size_t k = 0; k < par.size(); ++k) (fail[k] ? ser : ok).push_back(par[k]);
+        if (run_serial(ser) || run_cum(need_prep)) { free_all(); return -1; }
+        ser.clear();
+        if (!ok.empty()) {
+            // the sequences that stand: compact list (fail flags restart at 0)
+            cudaMemcpyAsync(d_list, ok.data(), sizeof(int32_t) * ok.size(), cudaMemcpyHostToDevice, stream);
+            cudaMemsetAsync(d_fail, 0, sizeof(int32_t) * ok.size(), stream);
+            a.n_seqs = (int32_t)ok.size();
+            cudaFuncSetAttribute(dfl_alone_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DflAloneSmem));
+            dfl_alone_kernel<<<(unsigned)std::min<size_t>(ok.size(), 148 * 8), DFL_ALONE_THREADS, sizeof(DflAloneSmem), stream>>>(
+                c, a, level, st.d_F[li], FQ, st.d_ckpt[li], cp);
+            ++*launches;
+            fail.assign(ok.size(), 0);
+            if (cudaGetLastError() != cudaSuccess ||
+                cudaMemcpyAsync(fail.data(), d_fail, sizeof(int32_t) * ok.size(), cudaMemcpyDeviceToHost, stream) != cudaSuccess ||
+                cudaStreamSynchronize(stream) != cudaSuccess) { free_all(); err = "dfl_alone_kernel failed"; return -1; }
+            std::vector<int32_t> redo;
+            for (size_t k = 0; k < ok.size(); ++k) if (fail[k]) redo.push_back(ok[k]);
+            st.parallel_prep_seqs += (int64_t)(ok.size() - redo.size());
+            if (run_serial(redo) || run_cum(redo)) { free_all(); return -1; }
+        }
+        free_all();
+    } else {
+        if (run_serial(ser) || run_cum(need_prep)) return -1;
+    }
+    for (int32_t i : need_prep) { st.have_prep[li][i] = 1; st.have_ckpt[li][i] = 1; }
     return 0;
 }
 
@@ -2243,7 +2642,7 @@ static int deflate_import_prefix(DeflateState &st, const DeflateCorpus &dc, int 
                                  const DflPrefixRecord *in, cudaStream_t stream, std::string &err)
 {
     const int li = level == 9 ? 0 : 1;
-    if (deflate_ensure_alloc(st, dc, level, stream, err)) return -1;
+    if (deflate_ensure_x(st, dc, level, stream, err)) return -1;
     for (int64_t k = 0; k < n; ++k) {
         const int32_t i = seqs[k];
         if (i < 0 || i >= dc.n_seqs) { err = "deflate_import_prefix: sequence index out of range"; return -1; }
@@ -2256,312 +2655,278 @@ static int deflate_import_prefix(DeflateState &st, const DeflateCorpus &dc, int 
     return 0;
 }
 
+// pair jobs (all, or the listed subset) through the junction / parse batches; sizes land at d_out[job]
+static int deflate_pairs(DeflateState &st, const DeflateCorpus &dc, int level, const int32_t *xs, const int32_t *ys,
+                         int64_t n_jobs, const std::vector<int64_t> *subset, int kind, size_t batch, int64_t *d_out,
+                         cudaStream_t stream, int64_t *launches, std::string &err)
+{
+    const int li = level == 9 ? 0 : 1;
+    uint32_t *FQ = level != 9 ? st.d_FQ : nullptr;
+    const int64_t total = subset ? (int64_t)subset->size() : n_jobs;
+    if (!total) return 0;
+    const int nbuf = total > (int64_t)batch ? 2 : 1;
+    const int parse_blocks = (int)std::min<size_t>(DFL_PARSE_BLOCKS, (batch + DFL_PARSE_THREADS - 1) / DFL_PARSE_THREADS);
+    for (int k = 0; k < nbuf; ++k) {
+        if (st.scratch_n[k] < (size_t)parse_blocks * DFL_PARSE_THREADS) {
+            dfl_free(st, st.d_scratch2[k]); st.scratch_n[k] = 0;
+            DCK(dfl_malloc(st, 3, &st.d_scratch2[k], sizeof(DflTrees) * (size_t)parse_blocks * DFL_PARSE_THREADS));
+            st.scratch_n[k] = (size_t)parse_blocks * DFL_PARSE_THREADS;
+        }
+        if (st.fj_pairs[k] < batch) {
+            dfl_free(st, st.d_FJ2[k]); dfl_free(st, st.d_FJQ2[k]); dfl_free(st, st.d_pairs2[k]); dfl_free(st, st.d_jobs2[k]);
+            st.fj_pairs[k] = 0;
+            DCK(dfl_malloc(st, 3, &st.d_FJ2[k], sizeof(uint32_t) * batch * DFL_JSTRIDE));
+            DCK(dfl_malloc(st, 3, &st.d_pairs2[k], sizeof(DflPair) * batch));
+            DCK(dfl_malloc(st, 3, &st.d_jobs2[k], sizeof(DflJob) * batch));
+            st.fj_pairs[k] = batch;
+        }
+        if (FQ && !st.d_FJQ2[k]) DCK(dfl_malloc(st, 3, &st.d_FJQ2[k], sizeof(uint32_t) * st.fj_pairs[k] * DFL_JSTRIDE));
+    }
+    DCK(cudaFuncSetAttribute(dfl_parse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)(DFL_PARSE_THREADS * sizeof(DflCompactTrees))));
+    if (!st.stream2) {
+        // the parse kernel is a few long-running, latency-bound CTAs: give it priority over the junction kernel's
+        // many short blocks, which would otherwise keep every SM full until they are all done
+        int prio_lo = 0, prio_hi = 0;
+        DCK(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
+        DCK(cudaStreamCreateWithPriority(&st.stream2, cudaStreamNonBlocking, prio_hi));
+        for (int k = 0; k < 2; ++k) {
+            DCK(cudaEventCreateWithFlags(&st.ev_j[k], cudaEventDisableTiming));
+            DCK(cudaEventCreateWithFlags(&st.ev_p[k], cudaEventDisableTiming));
+        }
+        DCK(dfl_malloc(st, 3, &st.d_counter2, 2 * sizeof(unsigned long long)));
+    }
+    const DflCorpus c = deflate_corpus(st, dc, li);
+    const DflCanonPool cp{st.d_sym_end[li], st.d_sym_code[li], st.d_cum[li], st.d_soff, st.d_cap, st.d_roff, st.d_nsym[li],
+                          st.d_seq_size[li]};
+    cudaEvent_t e0 = st.ev_t[0], e1 = st.ev_t[1];
+    std::vector<DflJob> jobs;
+    std::vector<DflPair> pairs;
+    NvtxRange nvtx_("snacc_b200: deflate pair batches (junction tables + pair parses)");
+    // measured: the junction kernel and the parse kernel running side by side (st.stream2) take 10 % longer
+    // than one after the other -- each fills the SMs on its own (registers / shared memory) -- so the second
+    // stream is only used when asked for; the double buffers still let the host prepare batch b+1 early
+    cudaStream_t pstream = getenv("SNACC_DFL_OVERLAP") ? st.stream2 : stream;
+    DCK(cudaEventRecord(st.ev_j[0], stream));                  // everything queued so far (prep) precedes the parses
+    DCK(cudaStreamWaitEvent(st.stream2, st.ev_j[0], 0));
+    int64_t nbatch = 0;
+    for (int64_t b0 = 0; b0 < total; b0 += (int64_t)batch, ++nbatch) {
+        const int k2 = (int)(nbatch & 1);
+        const int64_t nb = std::min<int64_t>((int64_t)batch, total - b0);
+        pairs.resize((size_t)nb); jobs.resize((size_t)nb);
+        for (int64_t k = 0; k < nb; ++k) {
+            const int64_t j = subset ? (*subset)[b0 + k] : b0 + k;
+            pairs[k] = DflPair{xs[j], ys[j]};
+            jobs[k] = DflJob{xs[j], ys[j], kind, (int32_t)k, j};
+        }
+        if (nbatch >= 2) DCK(cudaStreamWaitEvent(stream, st.ev_p[k2], 0));   // buffer k2 is free again
+        DCK(cudaMemcpyAsync(st.d_pairs2[k2], pairs.data(), sizeof(DflPair) * nb, cudaMemcpyHostToDevice, stream));
+        DCK(cudaMemcpyAsync(st.d_jobs2[k2], jobs.data(), sizeof(DflJob) * nb, cudaMemcpyHostToDevice, stream));
+        DCK(cudaEventRecord(e0, stream));
+        {
+            dim3 grid((DFL_JSTRIDE + 255) / 256, (unsigned)std::min<int64_t>(nb, 4096));
+            dfl_junction_kernel<<<grid, 256, 0, stream>>>(c, st.d_pairs2[k2], (int32_t)nb, level, st.d_F[li], FQ, st.d_FJ2[k2],
+                                                          FQ ? st.d_FJQ2[k2] : nullptr, st.junction_impl);
+        }
+        if (cudaGetLastError() != cudaSuccess) { err = "junction kernel launch failed"; return -1; }
+        DCK(cudaEventRecord(e1, stream));
+        DCK(cudaEventRecord(st.ev_j[k2], stream));
+        DCK(cudaStreamWaitEvent(pstream, st.ev_j[k2], 0));
+        DCK(cudaMemsetAsync(st.d_counter2 + k2, 0, sizeof(unsigned long long), pstream));
+        const int blocks = (int)std::min<size_t>(((size_t)nb + DFL_PARSE_THREADS - 1) / DFL_PARSE_THREADS, parse_blocks);
+        dfl_parse_kernel<<<blocks, DFL_PARSE_THREADS, DFL_PARSE_THREADS * sizeof(DflCompactTrees), pstream>>>(c, st.d_jobs2[k2], nb, level, st.d_F[li], FQ, st.d_FJ2[k2],
+                                                                      FQ ? st.d_FJQ2[k2] : nullptr, st.d_ckpt[li], cp,
+                                                                      st.d_scratch2[k2], st.d_counter2 + k2, d_out);
+        if (cudaGetLastError() != cudaSuccess) { err = "dfl_parse_kernel launch failed"; return -1; }
+        DCK(cudaEventRecord(st.ev_p[k2], pstream));
+        *launches += 2;
+        // the host buffers are reused for the next batch: wait until this batch's uploads are done (the
+        // kernels of the previous batch keep the GPU busy meanwhile)
+        DCK(cudaEventSynchronize(st.ev_j[k2]));
+        float ms = 0.f;
+        DCK(cudaEventElapsedTime(&ms, e0, e1));
+        st.main_ms += ms;                                  // the junction kernel is the dominant one
+    }
+    DCK(cudaStreamSynchronize(st.stream2));
+    DCK(cudaStreamSynchronize(stream));
+    if (kind != 2) return 0;
+    // jobs whose shortcut met a block that might be stored (-2): full serial parse
+    std::vector<int64_t> h_out((size_t)n_jobs), redo;
+    DCK(cudaMemcpyAsync(h_out.data(), d_out, sizeof(int64_t) * n_jobs, cudaMemcpyDeviceToHost, stream));
+    DCK(cudaStreamSynchronize(stream));
+    for (int64_t k = 0; k < total; ++k) {
+        const int64_t j = subset ? (*subset)[k] : k;
+        if (h_out[j] == -2) redo.push_back(j);
+    }
+    st.serial_jobs += (int64_t)redo.size();
+    return redo.empty() ? 0 : deflate_pairs(st, dc, level, xs, ys, n_jobs, &redo, 4, batch, d_out, stream, launches, err);
+}
+
+// sizes of the raw deflate streams of the jobs (x alone when ys == nullptr) into d_out[0..n_jobs)
 static int deflate_run(DeflateState &st, const DeflateCorpus &dc, int level, const int32_t *xs, const int32_t *ys,
                        const int32_t *d_xs, const int32_t *, int64_t n_jobs, int64_t *d_out, cudaStream_t stream,
                        int64_t, int64_t *launches, std::string &err)
 {
     const int li = level == 9 ? 0 : 1;
     const int32_t ns = dc.n_seqs;
-    if (deflate_ensure_alloc(st, dc, level, stream, err)) return -1;
-    uint32_t *FQ = level != 9 ? st.d_FQ : nullptr;
-    DflCorpus c{dc.d_corpus, dc.d_off, dc.d_len, st.d_poff, st.d_order, st.d_bstart, st.d_head_order, st.d_head_visit[li],
-                st.d_tail_cnt, st.d_tail6_order, st.d_tail6_start, nullptr, st.d_bstart6, st.d_ifrom};
-    DflCanonPool cp{st.d_sym_end[li], st.d_sym_code[li], st.d_cum[li], st.d_soff, st.d_cap, st.d_roff, st.d_nsym[li],
-                    st.d_seq_size[li]};
+    st.main_ms = 0.0; st.serial_jobs = 0; st.bands = 0; st.prepared_seqs = 0; st.parallel_prep_seqs = 0;
+    st.peak = st.live[0] + st.live[1] + st.live[2] + st.live[3];
 
-    // ---- per-sequence state the jobs need: index, F (this level), and the parse of the sequence alone
-    //      (size, checkpoint, canonical symbol stream) ----
-    std::vector<int32_t> need_idx, need_f, need_prep;
-    {
-        // role of every sequence in this call: bit 0 = x of a pair stream or a single (needs its index -- the junction
-        // walk reads x's buckets -- and its x-side product, own or imported), bit 1 = y of a pair stream (needs its
-        // index, match table and the parse of the sequence alone: canonical stream, head visits)
-        std::vector<uint8_t> used(ns, 0);
-        for (int64_t k = 0; k < n_jobs; ++k) { used[xs[k]] |= 1; if (ys) used[ys[k]] |= 2; }
-        for (int32_t i = 0; i < ns; ++i) {
-            if (!used[i]) continue;
-            const bool full = (used[i] & 2) || !st.have_ckpt[li][i];
-            // indexed: 0 none, 1 the last DFL_XTAIL positions only (enough for the x of a pair stream), 2 whole sequence
-            if (!full) {
-                if (ys && !st.indexed[i]) {
-                    need_idx.push_back(i); st.indexed[i] = 1; st.have_F[0][i] = st.have_F[1][i] = 0;
-                    st.h_ifrom[i] = st.use_tail_index && dc.h_len[i] > DFL_XTAIL ? dc.h_len[i] - DFL_XTAIL : 0;
-                    if (!st.h_ifrom[i]) st.indexed[i] = 2;
-                }
-                continue;
-            }
-            if (st.indexed[i] < 2) { need_idx.push_back(i); st.indexed[i] = 2; st.h_ifrom[i] = 0; st.have_F[0][i] = st.have_F[1][i] = 0; }
-            if (!st.have_F[li][i]) { need_f.push_back(i); st.have_F[li][i] = 1; st.have_prep[li][i] = 0; }
-            if (!st.have_prep[li][i]) { need_prep.push_back(i); st.have_prep[li][i] = 1; st.have_ckpt[li][i] = 1; }
-        }
+    // ---- roles.  x of a pair stream or a single: its record (own parse or imported) and, for pair streams, an
+    //      index; y of a pair stream: the full preparation; a sequence without a record gets the full preparation
+    //      once to produce it ----
+    const bool x_ready = st.n_seqs == ns && st.d_xoff && st.d_ckpt[li];     // (records outlive a new x index layout)
+    std::vector<uint8_t> used(ns, 0);
+    for (int64_t k = 0; k < n_jobs; ++k) { used[xs[k]] |= 1; if (ys) used[ys[k]] |= 2; }
+    std::vector<int32_t> full, ylist_all, no_rec, xpair;
+    for (int32_t i = 0; i < ns; ++i) {
+        if (!used[i]) continue;
+        const bool rec = x_ready && st.have_ckpt[li][i];
+        if (!rec) no_rec.push_back(i);
+        if (used[i] & 2) ylist_all.push_back(i);
+        if ((used[i] & 2) || !rec) full.push_back(i);
+        if (ys && (used[i] & 1)) xpair.push_back(i);
     }
-    uint32_t max_len = 0;
-    for (int32_t i : need_f) max_len = std::max(max_len, dc.h_len[i]);
-    if (!need_idx.empty()) {
-        NvtxRange nvtx_("snacc_b200: deflate index (radix sort, head/tail packs)");
-        int32_t *d_list = nullptr;
-        if (dfl_upload(err, stream, need_idx, &d_list)) return -1;
-        DCK(cudaMemcpyAsync(st.d_ifrom, st.h_ifrom.data(), sizeof(uint32_t) * st.h_ifrom.size(), cudaMemcpyHostToDevice, stream));
-        // the F slices of this level double as sort scratch; they are recomputed right below
-        for (size_t a0 = 0; a0 < need_idx.size(); a0 += 64) {
-            std::vector<int32_t> part(need_idx.begin() + a0, need_idx.begin() + std::min(need_idx.size(), a0 + 64));
-            if (dfl_build_index<0>(st, c, part, dc.h_len, st.d_F[li], stream, launches, err)) return -1;
-        }
-        DCK(cudaFuncSetAttribute(dfl_head_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(DFL_HASH * 4)));
-        dfl_head_kernel<<<(unsigned)std::min<size_t>(need_idx.size(), 148), 1024, DFL_HASH * 4, stream>>>(
-            c, d_list, (int32_t)need_idx.size());
-        DCK(cudaGetLastError());
-        const int t6_smem = (int)(DFL_H6 * 4 + DFL_T6 * 2);
-        DCK(cudaFuncSetAttribute(dfl_tail6_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, t6_smem));
-        dfl_tail6_kernel<<<(unsigned)std::min<size_t>(need_idx.size(), 148 * 2), 32, t6_smem, stream>>>(c, d_list, (int32_t)need_idx.size());
-        DCK(cudaGetLastError());
-        *launches += 3;
-        DCK(cudaStreamSynchronize(stream));
-        cudaFree(d_list);
+
+    // ---- memory plan (device bytes; free memory read now: the device is shared) ----
+    size_t free0 = 0, total0 = 0;
+    DCK(cudaMemGetInfo(&free0, &total0));
+    const size_t batch = ys ? std::min<size_t>(DFL_BATCH, (size_t)n_jobs) : 0;
+    uint64_t x_need = 0;                                              // x side still to allocate
+    if (!(st.n_seqs == ns && st.d_xoff)) x_need += (uint64_t)ns * dfl_xbytes_fixed();
+    if (!(st.n_seqs == ns && st.d_xoff && st.x_whole == (st.use_tail_index ? 0 : 1)))
+        for (int32_t i = 0; i < ns; ++i) x_need += 4 * dfl_xslot(dc.h_len[i], st.use_tail_index ? 0 : 1);
+    if (!(st.n_seqs == ns && st.d_ckpt[li])) x_need += (uint64_t)ns * dfl_xbytes_level();
+    uint32_t max_len = 0; uint64_t y_all = 0, y_max = 0;
+    for (int32_t i : full) { const uint64_t b = dfl_ybytes(dc.h_len[i], level); y_all += b; y_max = std::max(y_max, b); max_len = std::max(max_len, dc.h_len[i]); }
+    uint64_t work = 0;
+    if (ys) {
+        const uint64_t nbuf = (uint64_t)n_jobs > batch ? 2 : 1;
+        const uint64_t threads = std::min<uint64_t>(DFL_PARSE_BLOCKS, (batch + DFL_PARSE_THREADS - 1) / DFL_PARSE_THREADS) * DFL_PARSE_THREADS;
+        work += nbuf * (batch * ((uint64_t)DFL_JSTRIDE * 4 * (level == 9 ? 1 : 2) + sizeof(DflPair) + sizeof(DflJob)) + threads * sizeof(DflTrees));
+        uint64_t sum = 0, big = 0;                                      // x index sort scratch, as deflate_build_x sizes it
+        for (int32_t i : xpair) { const uint64_t v = dfl_xslot(dc.h_len[i], st.use_tail_index ? 0 : 1); sum += v; big = std::max(big, v); }
+        work += 4 * (std::max(big, std::min<uint64_t>(sum, (uint64_t)DFL_INDEX_GROUP * DFL_XTAIL)) + 16);
     }
-    if (!need_f.empty()) {
-        NvtxRange nvtx_("snacc_b200: deflate match tables");
-        // level 9: runs of sequences whose index slices fit the window buffer get a transient 6-byte index first
-        // (dfl_match_word); level 6 always walks the chain (its limit of 128 binds everywhere on DNA)
-        const bool i6 = st.use_index6 && level == 9;
-        const uint64_t cap = 192ull << 20;                                     // entries: 768 MB
-        if (i6 && !st.d_order6) { DCK(cudaMalloc(&st.d_order6, sizeof(uint32_t) * (cap + 16))); st.order6_cap = cap; }
-        size_t a = 0;
-        while (a < need_f.size()) {
-            size_t b = a + 1;
-            const uint64_t first = st.h_poff[need_f[a]];
-            auto end_of = [&](int32_t i) { return st.h_poff[i] + (((uint64_t)dc.h_len[i] + 7) & ~7ull); };
-            while (b < need_f.size() && b - a < 64 && (!i6 || end_of(need_f[b]) - first <= cap)) ++b;
-            const bool fits = i6 && end_of(need_f[b - 1]) - first <= cap;      // (a single sequence longer than the buffer: no index)
-            std::vector<int32_t> part(need_f.begin() + a, need_f.begin() + b);
-            int32_t *d_list = nullptr;
-            if (dfl_upload(err, stream, part, &d_list)) return -1;
-            DflCorpus cm = c;
-            if (fits) {
-                cm.order6 = st.d_order6 - first;                               // addressed like `order`: + poff[sq]
-                if (dfl_build_index<1>(st, cm, part, dc.h_len, st.d_F[li], stream, launches, err)) return -1;
-            }
-            uint32_t mx = 0;
-            for (int32_t i : part) mx = std::max(mx, dc.h_len[i]);
-            dim3 grid(std::max(1u, std::min((mx + 255) / 256, 4096u)), (unsigned)part.size());
-            dfl_match_kernel<<<grid, 256, 0, stream>>>(cm, d_list, (int32_t)part.size(), level, st.d_F[li], FQ);
-            DCK(cudaGetLastError());
-            ++*launches;
-            DCK(cudaStreamSynchronize(stream));
-            cudaFree(d_list);
-            a = b;
-        }
+    if (!full.empty()) {
+        if (st.use_index6 && level == 9) work += 4 * (std::min<uint64_t>(DFL_ORDER6_CAP, y_all) + 16);
+        work += 4ull * DFL_INDEX_GROUP * 256 * std::max(1u, dfl_rx_tiles(max_len));
     }
-    // ---- parse jobs ----
-    // working buffers are sized for the jobs of this call (a one-pair call -- the compressed_size() shim -- must not
-    // reserve the 2 x 6.3 GB a full batch needs) and grow on demand
-    const size_t batch = ys ? std::min<size_t>(DFL_BATCH, (((size_t)n_jobs + 63) / 64) * 64) : 64;
-    const int parse_blocks = (int)std::min<size_t>(DFL_PARSE_BLOCKS, batch / DFL_PARSE_THREADS);
-    if (ys && st.scratch_n < (size_t)parse_blocks * DFL_PARSE_THREADS) {
-        for (int k = 0; k < 2; ++k) { cudaFree(st.d_scratch2[k]); st.d_scratch2[k] = nullptr; }
-        st.scratch_n = 0;
-        for (int k = 0; k < 2; ++k) DCK(cudaMalloc(&st.d_scratch2[k], sizeof(DflTrees) * (size_t)parse_blocks * DFL_PARSE_THREADS));
-        st.scratch_n = (size_t)parse_blocks * DFL_PARSE_THREADS;
+    const uint64_t margin = (256ull << 20) + total0 / 100;           // allocator granularity, kernel stacks, the caller's epilogue
+    // pair-batch buffers of another shape than this call's are released now: what stays is what the call reuses.  A call
+    // without pair jobs leaves them alone and counts them as held.
+    if (ys) {
+        const size_t threads = std::min<size_t>(DFL_PARSE_BLOCKS, (batch + DFL_PARSE_THREADS - 1) / DFL_PARSE_THREADS) * DFL_PARSE_THREADS;
+        const bool same = st.fj_pairs[0] == batch && st.scratch_n[0] == threads && (st.d_FJ2[1] != nullptr) == ((size_t)n_jobs > batch) &&
+                          (st.d_FJ2[1] == nullptr || (st.fj_pairs[1] == batch && st.scratch_n[1] == threads)) &&
+                          (st.d_FJQ2[0] != nullptr) == (level != 9);
+        if (!same) deflate_free_batches(st);
     }
-    st.main_ms = 0.0;
-    st.serial_jobs = 0;
+    // y layout (dropped when the call needs another), preparation scratch (none between calls), batch buffers (above)
+    const uint64_t reusable = (uint64_t)st.live[1] + st.live[2] + (ys ? st.live[3] : 0);
+    const uint64_t avail = free0 + reusable;
+    const uint64_t fixed = x_need + work + margin;
+    uint64_t y_budget = avail > fixed ? avail - fixed : 0;
+    if (st.band_bytes > 0) y_budget = std::min<uint64_t>(y_budget, (uint64_t)st.band_bytes);
+    if (!full.empty() && y_max > y_budget) {
+        char b_[512];
+        snprintf(b_, sizeof b_, "deflate: the x side of %d sequences, the working buffers and one y need %.3f GB of device memory "
+                 "(%llu bytes; y layout capped at %llu bytes), %llu bytes are free",
+                 ns, (double)(fixed + y_max) / 1e9, (unsigned long long)(fixed + y_max),
+                 (unsigned long long)(st.band_bytes > 0 ? (uint64_t)st.band_bytes : avail), (unsigned long long)avail);
+        err = b_;
+        return SNACC_ERR_TOO_LARGE;
+    }
+    if (deflate_ensure_x(st, dc, level, stream, err)) return -1;
     if (!st.ev_t[0]) { DCK(cudaEventCreate(&st.ev_t[0])); DCK(cudaEventCreate(&st.ev_t[1])); }   // owned by the state: no leak on error paths
-    cudaEvent_t e0 = st.ev_t[0], e1 = st.ev_t[1];
-    int rc = 0;
-    if (!need_prep.empty()) {
-        NvtxRange nvtx_("snacc_b200: deflate sequence parses (sizes, checkpoints, canonical streams)");
-        // long sequences: chunks in parallel (dfl_chunk_*_kernel), then cumulative rows, then dfl_alone_kernel; the
-        // others -- and whatever the parallel path gives up on -- take the serial kernel
-        std::vector<int32_t> par, ser;
-        for (int32_t i : need_prep) (st.use_parallel_prep && dc.h_len[i] >= DFL_PAR_MIN ? par : ser).push_back(i);
-        auto run_serial = [&](const std::vector<int32_t> &list) -> int {
-            if (list.empty()) return 0;
-            int32_t *d_list = nullptr;
-            if (dfl_upload(err, stream, list, &d_list)) return -1;
-            DCK(cudaFuncSetAttribute(dfl_prep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DflPrepSmem)));
-            dfl_prep_kernel<<<(unsigned)std::min<size_t>(list.size(), 148 * 5), DFL_PREP_THREADS, sizeof(DflPrepSmem), stream>>>(
-                c, d_list, (int32_t)list.size(), level, st.d_F[li], FQ, st.d_ckpt[li], cp);
-            DCK(cudaGetLastError());
-            ++*launches;
-            DCK(cudaStreamSynchronize(stream));
-            cudaFree(d_list);
-            return 0;
-        };
-        auto run_cum = [&](const std::vector<int32_t> &list) -> int {
-            if (list.empty()) return 0;
-            int32_t *d_list = nullptr;
-            if (dfl_upload(err, stream, list, &d_list)) return -1;
-            uint32_t max_rows = 1;
-            for (int32_t i : list) max_rows = std::max(max_rows, dc.h_len[i] / 4 / DFL_CUM_G + 8);
-            dim3 grid(std::min(max_rows, 2048u), (unsigned)std::min<size_t>(list.size(), 64));
-            dfl_cum_chunk_kernel<<<grid, 64, 0, stream>>>(cp, d_list, (int32_t)list.size());
-            dfl_cum_scan_kernel<<<(unsigned)std::min<size_t>(list.size(), 148 * 4), DFL_CUM_W, 0, stream>>>(
-                cp, d_list, (int32_t)list.size());
-            DCK(cudaGetLastError());
-            *launches += 2;
-            DCK(cudaStreamSynchronize(stream));
-            cudaFree(d_list);
-            return 0;
-        };
-        st.parallel_prep_seqs = 0;
-        if (!par.empty()) {
-            // per-chunk scratch of the listed sequences (2 x 128 B of bitmaps + 12 B per 8 KiB chunk)
-            std::vector<uint64_t> coff(par.size() + 1, 0);
-            uint32_t max_k = 1;
-            for (size_t k = 0; k < par.size(); ++k) {
-                const uint32_t K = dfl_chunk_count(dc.h_len[par[k]]);
-                coff[k + 1] = coff[k] + K; max_k = std::max(max_k, K);
+
+    bool in_layout = !st.ylist.empty();
+    for (int32_t i : full) in_layout = in_layout && st.h_yslot[i] != DFL_NONE;
+    if (in_layout) {
+        // the layout holds the sequences (it may hold more): keep it only if all of it, with this level's arrays when they
+        // are missing, fits the budget -- a kept layout is not released
+        uint64_t lb = 0;
+        if (!st.d_F[li])
+            for (int32_t i : st.ylist) {
+                const uint64_t cap = dfl_canon_cap(dc.h_len[i]);
+                lb += dfl_pad8(dc.h_len[i]) * 4 * (level == 9 || st.d_FQ ? 1 : 2) + 2ull * DFL_JY + cap * 6 + (cap / DFL_CUM_G + 1) * DFL_CUM_W * 4;
             }
-            const uint64_t tot = coff.back();
-            int32_t *d_list = nullptr; uint64_t *d_coff = nullptr; uint32_t *d_w = nullptr; int32_t *d_fail = nullptr;
-            if (dfl_upload(err, stream, par, &d_list)) return -1;
-            auto free_all = [&]() { cudaFree(d_list); cudaFree(d_coff); cudaFree(d_w); cudaFree(d_fail); };
-            if (cudaMalloc(&d_coff, sizeof(uint64_t) * coff.size()) != cudaSuccess ||
-                cudaMalloc(&d_w, sizeof(uint32_t) * tot * (2 * DFL_CHUNK_WORDS + 3)) != cudaSuccess ||
-                cudaMalloc(&d_fail, sizeof(int32_t) * par.size()) != cudaSuccess) { free_all(); err = "cudaMalloc (chunk scratch) failed"; return -1; }
-            cudaMemcpyAsync(d_coff, coff.data(), sizeof(uint64_t) * coff.size(), cudaMemcpyHostToDevice, stream);
-            cudaMemsetAsync(d_fail, 0, sizeof(int32_t) * par.size(), stream);
-            DflChunkArgs a{d_list, d_coff, (int32_t)par.size(), d_w, d_w + tot * DFL_CHUNK_WORDS, d_w + tot * 2 * DFL_CHUNK_WORDS,
-                           d_w + tot * (2 * DFL_CHUNK_WORDS + 1), d_w + tot * (2 * DFL_CHUNK_WORDS + 2), d_fail};
-            dim3 grid((max_k + 127) / 128, (unsigned)std::min<size_t>(par.size(), 65535));
-            dfl_chunk_scan_kernel<<<grid, 128, 0, stream>>>(c, a, level, st.d_F[li], FQ);
-            dfl_chunk_pass_kernel<1><<<grid, 128, 0, stream>>>(c, a, level, st.d_F[li], FQ, cp);
-            dfl_chunk_offsets_kernel<<<(unsigned)((par.size() + 63) / 64), 64, 0, stream>>>(c, a, cp);
-            dfl_chunk_pass_kernel<2><<<grid, 128, 0, stream>>>(c, a, level, st.d_F[li], FQ, cp);
-            *launches += 4;
-            std::vector<int32_t> fail(par.size(), 0);
-            if (cudaGetLastError() != cudaSuccess ||
-                cudaMemcpyAsync(fail.data(), d_fail, sizeof(int32_t) * par.size(), cudaMemcpyDeviceToHost, stream) != cudaSuccess ||
-                cudaStreamSynchronize(stream) != cudaSuccess) { free_all(); err = "deflate chunk kernels failed"; return -1; }
-            std::vector<int32_t> ok;
-            for (size_t k = 0; k < par.size(); ++k) (fail[k] ? ser : ok).push_back(par[k]);
-            if (run_serial(ser) || run_cum(need_prep)) { free_all(); return -1; }
-            ser.clear();
-            if (!ok.empty()) {
-                // the sequences that stand: compact list (fail flags restart at 0)
-                cudaMemcpyAsync(d_list, ok.data(), sizeof(int32_t) * ok.size(), cudaMemcpyHostToDevice, stream);
-                cudaMemsetAsync(d_fail, 0, sizeof(int32_t) * ok.size(), stream);
-                a.n_seqs = (int32_t)ok.size();
-                cudaFuncSetAttribute(dfl_alone_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DflAloneSmem));
-                dfl_alone_kernel<<<(unsigned)std::min<size_t>(ok.size(), 148 * 8), DFL_ALONE_THREADS, sizeof(DflAloneSmem), stream>>>(
-                    c, a, level, st.d_F[li], FQ, st.d_ckpt[li], cp);
-                ++*launches;
-                fail.assign(ok.size(), 0);
-                if (cudaGetLastError() != cudaSuccess ||
-                    cudaMemcpyAsync(fail.data(), d_fail, sizeof(int32_t) * ok.size(), cudaMemcpyDeviceToHost, stream) != cudaSuccess ||
-                    cudaStreamSynchronize(stream) != cudaSuccess) { free_all(); err = "dfl_alone_kernel failed"; return -1; }
-                std::vector<int32_t> redo;
-                for (size_t k = 0; k < ok.size(); ++k) if (fail[k]) redo.push_back(ok[k]);
-                st.parallel_prep_seqs = (int64_t)(ok.size() - redo.size());
-                if (run_serial(redo) || run_cum(redo)) { free_all(); return -1; }
-            }
-            free_all();
-        } else {
-            if (run_serial(ser) || run_cum(need_prep)) return -1;
-        }
+        in_layout = st.live[1] + lb <= y_budget;
     }
-    if (rc) { /* fall through to cleanup */ }
-    else if (!ys) {
-        dfl_gather_sizes_kernel<<<(unsigned)((n_jobs + 255) / 256), 256, 0, stream>>>(st.d_seq_size[li], d_xs, n_jobs, d_out);
-        if (cudaGetLastError() != cudaSuccess) { err = "dfl_gather_sizes_kernel launch failed"; rc = -1; }
-        ++*launches;
+    bool banded = false;
+    if (in_layout || y_all <= y_budget || full.empty()) {
+        // ---- one band: the whole y state of the call in one layout, which stays resident for later calls ----
+        st.bands = 1;
+        if (!full.empty()) {
+            if (!in_layout) { if (deflate_set_layout(st, dc, level, full, stream, err)) return -1; }
+            else if (deflate_ensure_y_level(st, level, err)) return -1;
+            if (deflate_prepare_y(st, dc, level, full, stream, launches, err)) return -1;
+        }
+        if (ys) {
+            std::vector<int32_t> need_x;
+            for (int32_t i : xpair) if (!st.yindexed[i] && !st.xindexed[i]) need_x.push_back(i);
+            if (deflate_build_x(st, dc, li, need_x, stream, launches, err)) return -1;
+            if (deflate_upload_ix(st, stream, err)) return -1;
+            if (deflate_pairs(st, dc, level, xs, ys, n_jobs, nullptr, st.use_canon ? 2 : 4, batch, d_out, stream, launches, err)) return -1;
+        }
     } else {
-        // pairs in batches, double buffered: the junction tables of batch b+1 are computed on `stream` while the
-        // pair streams of batch b are parsed on st.stream2 (a latency-bound kernel with one thread per stream)
-        if (st.fj_pairs < batch) {
-            for (int k = 0; k < 2; ++k) {
-                cudaFree(st.d_FJ2[k]); cudaFree(st.d_pairs2[k]); cudaFree(st.d_jobs2[k]); cudaFree(st.d_FJQ2[k]);
-                st.d_FJ2[k] = st.d_FJQ2[k] = nullptr; st.d_pairs2[k] = nullptr; st.d_jobs2[k] = nullptr;
+        // ---- bands: the y layout of each band holds what fits in y_budget; afterwards only the x side stays ----
+        banded = true;
+        deflate_drop_y(st);
+        deflate_free_batches(st);
+        auto cut = [&](const std::vector<int32_t> &list) {
+            std::vector<std::vector<int32_t>> out;
+            uint64_t acc = 0;
+            for (int32_t i : list) {
+                const uint64_t b = dfl_ybytes(dc.h_len[i], level);
+                if (out.empty() || acc + b > y_budget) { out.emplace_back(); acc = 0; }
+                out.back().push_back(i); acc += b;
             }
-            st.fj_pairs = 0;
-            for (int k = 0; k < 2; ++k) {
-                DCK(cudaMalloc(&st.d_FJ2[k], sizeof(uint32_t) * batch * DFL_JSTRIDE));
-                DCK(cudaMalloc(&st.d_pairs2[k], sizeof(DflPair) * batch));
-                DCK(cudaMalloc(&st.d_jobs2[k], sizeof(DflJob) * batch));
-            }
-            st.fj_pairs = batch;
-        }
-        if (FQ && !st.d_FJQ2[0])
-            for (int k = 0; k < 2; ++k) DCK(cudaMalloc(&st.d_FJQ2[k], sizeof(uint32_t) * batch * DFL_JSTRIDE));
-        DCK(cudaFuncSetAttribute(dfl_parse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)(DFL_PARSE_THREADS * sizeof(DflCompactTrees))));
-        if (!st.stream2) {
-            // the parse kernel is a few long-running, latency-bound CTAs: give it priority over the junction kernel's
-            // many short blocks, which would otherwise keep every SM full until they are all done
-            int prio_lo = 0, prio_hi = 0;
-            DCK(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
-            DCK(cudaStreamCreateWithPriority(&st.stream2, cudaStreamNonBlocking, prio_hi));
-            for (int k = 0; k < 2; ++k) {
-                DCK(cudaEventCreateWithFlags(&st.ev_j[k], cudaEventDisableTiming));
-                DCK(cudaEventCreateWithFlags(&st.ev_p[k], cudaEventDisableTiming));
-            }
-            DCK(cudaMalloc(&st.d_counter2, 2 * sizeof(unsigned long long)));
-        }
-        std::vector<DflJob> jobs;
-        std::vector<DflPair> pairs;
-        auto run_pairs = [&](const std::vector<int64_t> *subset, int kind) -> int {
-            NvtxRange nvtx_("snacc_b200: deflate pair batches (junction tables + pair parses)");
-            const int64_t total = subset ? (int64_t)subset->size() : n_jobs;
-            // measured: the junction kernel and the parse kernel running side by side (st.stream2) take 10 % longer
-            // than one after the other -- each fills the SMs on its own (registers / shared memory) -- so the second
-            // stream is only used when asked for; the double buffers still let the host prepare batch b+1 early
-            cudaStream_t pstream = getenv("SNACC_DFL_OVERLAP") ? st.stream2 : stream;
-            DCK(cudaEventRecord(st.ev_j[0], stream));                  // everything queued so far (prep) precedes the parses
-            DCK(cudaStreamWaitEvent(st.stream2, st.ev_j[0], 0));
-            int64_t nbatch = 0;
-            for (int64_t b0 = 0; b0 < total; b0 += (int64_t)batch, ++nbatch) {
-                const int k2 = (int)(nbatch & 1);
-                const int64_t nb = std::min<int64_t>((int64_t)batch, total - b0);
-                pairs.resize((size_t)nb); jobs.resize((size_t)nb);
-                for (int64_t k = 0; k < nb; ++k) {
-                    const int64_t j = subset ? (*subset)[b0 + k] : b0 + k;
-                    pairs[k] = DflPair{xs[j], ys[j]};
-                    jobs[k] = DflJob{xs[j], ys[j], kind, (int32_t)k, j};
-                }
-                if (nbatch >= 2) DCK(cudaStreamWaitEvent(stream, st.ev_p[k2], 0));   // buffer k2 is free again
-                DCK(cudaMemcpyAsync(st.d_pairs2[k2], pairs.data(), sizeof(DflPair) * nb, cudaMemcpyHostToDevice, stream));
-                DCK(cudaMemcpyAsync(st.d_jobs2[k2], jobs.data(), sizeof(DflJob) * nb, cudaMemcpyHostToDevice, stream));
-                DCK(cudaEventRecord(e0, stream));
-                {
-                    dim3 grid((DFL_JSTRIDE + 255) / 256, (unsigned)std::min<int64_t>(nb, 4096));
-                    dfl_junction_kernel<<<grid, 256, 0, stream>>>(c, st.d_pairs2[k2], (int32_t)nb, level, st.d_F[li], FQ, st.d_FJ2[k2],
-                                                                  FQ ? st.d_FJQ2[k2] : nullptr, st.junction_impl);
-                }
-                if (cudaGetLastError() != cudaSuccess) { err = "junction kernel launch failed"; return -1; }
-                DCK(cudaEventRecord(e1, stream));
-                DCK(cudaEventRecord(st.ev_j[k2], stream));
-                DCK(cudaStreamWaitEvent(pstream, st.ev_j[k2], 0));
-                DCK(cudaMemsetAsync(st.d_counter2 + k2, 0, sizeof(unsigned long long), pstream));
-                const int blocks = (int)std::min<size_t>(((size_t)nb + DFL_PARSE_THREADS - 1) / DFL_PARSE_THREADS, parse_blocks);
-                dfl_parse_kernel<<<blocks, DFL_PARSE_THREADS, DFL_PARSE_THREADS * sizeof(DflCompactTrees), pstream>>>(c, st.d_jobs2[k2], nb, level, st.d_F[li], FQ, st.d_FJ2[k2],
-                                                                              FQ ? st.d_FJQ2[k2] : nullptr, st.d_ckpt[li], cp,
-                                                                              st.d_scratch2[k2], st.d_counter2 + k2, d_out);
-                if (cudaGetLastError() != cudaSuccess) { err = "dfl_parse_kernel launch failed"; return -1; }
-                DCK(cudaEventRecord(st.ev_p[k2], pstream));
-                *launches += 2;
-                // the host buffers are reused for the next batch: wait until this batch's uploads are done (the
-                // kernels of the previous batch keep the GPU busy meanwhile)
-                DCK(cudaEventSynchronize(st.ev_j[k2]));
-                float ms = 0.f;
-                DCK(cudaEventElapsedTime(&ms, e0, e1));
-                st.main_ms += ms;                                  // the junction kernel is the dominant one
-            }
-            DCK(cudaStreamSynchronize(st.stream2));
-            DCK(cudaStreamSynchronize(stream));
-            return 0;
+            return out;
         };
-        rc = run_pairs(nullptr, st.use_canon ? 2 : 4);
-        if (!rc && st.use_canon) {
-            // jobs whose shortcut met a block that might be stored (-2): full serial parse
-            std::vector<int64_t> h_out((size_t)n_jobs), redo;
-            DCK(cudaMemcpyAsync(h_out.data(), d_out, sizeof(int64_t) * n_jobs, cudaMemcpyDeviceToHost, stream));
-            DCK(cudaStreamSynchronize(stream));
-            for (int64_t k = 0; k < n_jobs; ++k) if (h_out[k] == -2) redo.push_back(k);
-            st.serial_jobs = (int64_t)redo.size();
-            if (!redo.empty()) rc = run_pairs(&redo, 4);
+        // pass 0: the records of the sequences that have none
+        for (const auto &part : cut(no_rec)) {
+            ++st.bands;
+            if (deflate_set_layout(st, dc, level, part, stream, err)) return -1;
+            if (deflate_prepare_y(st, dc, level, part, stream, launches, err)) return -1;
+        }
+        deflate_drop_y(st);
+        if (ys) {
+            // pass 1: x index slices of every x, then the pair jobs band by band of their y, in the caller's job order
+            std::vector<int32_t> need_x;
+            for (int32_t i : xpair) if (!st.xindexed[i]) need_x.push_back(i);
+            if (deflate_build_x(st, dc, li, need_x, stream, launches, err)) return -1;
+            std::vector<int32_t> band_of(ns, -1);
+            const auto bands = cut(ylist_all);
+            for (size_t b = 0; b < bands.size(); ++b) for (int32_t i : bands[b]) band_of[i] = (int32_t)b;
+            std::vector<std::vector<int64_t>> jobs_of(bands.size());
+            for (int64_t k = 0; k < n_jobs; ++k) jobs_of[band_of[ys[k]]].push_back(k);
+            for (size_t b = 0; b < bands.size(); ++b) {
+                ++st.bands;
+                if (deflate_set_layout(st, dc, level, bands[b], stream, err)) return -1;
+                if (deflate_prepare_y(st, dc, level, bands[b], stream, launches, err)) return -1;
+                if (deflate_upload_ix(st, stream, err)) return -1;
+                if (deflate_pairs(st, dc, level, xs, ys, n_jobs, &jobs_of[b], st.use_canon ? 2 : 4, batch, d_out, stream, launches, err))
+                    return -1;
+            }
         }
     }
-    return rc;
+    if (!ys) {
+        dfl_gather_sizes_kernel<<<(unsigned)((n_jobs + 255) / 256), 256, 0, stream>>>(st.d_seq_size[li], d_xs, n_jobs, d_out);
+        if (cudaGetLastError() != cudaSuccess) { err = "dfl_gather_sizes_kernel launch failed"; return -1; }
+        ++*launches;
+    }
+    DCK(cudaStreamSynchronize(stream));
+    dfl_free(st, st.d_order6); st.order6_cap = 0;                  // preparation scratch: none between calls
+    dfl_free(st, st.d_rx_hist); st.rx_cap = 0;
+    dfl_free(st, st.d_xtmp); st.xtmp_cap = 0;
+    if (banded) {
+        // what stays is the x side: the caller's epilogue (snacc_ncd, a gather across ranks) needs the room
+        deflate_drop_y(st);
+        deflate_free_batches(st);
+        if (deflate_upload_ix(st, stream, err)) return -1;
+    }
+    return 0;
 }
 #undef DCK
 #endif  // __CUDACC__
