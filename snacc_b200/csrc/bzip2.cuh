@@ -9,6 +9,8 @@
 // against libbz2); the kernels (bz_*) compose those functions in parallel.
 #pragma once
 #include <stdint.h>
+#include <algorithm>
+#include <string>
 #include <vector>
 #include "common.cuh"
 
@@ -618,6 +620,222 @@ __global__ void bz_finish_kernel(const unsigned long long *__restrict__ job_bits
         if (use_prefix[k]) bits += (int64_t)seq_bits[xs[k]];
         out[k] = bz_stream_bytes(bits);
     }
+}
+
+
+// ---- host side (called from api.cu with the context lock held) ------------------------------------------------------
+// RLE1 of every sequence once per upload; then per call the host cuts every job into blocks (x's closed blocks once per
+// x, the rest of each job from x's open tail, the junction and RLE1(y)) and the blocks go through fixed-size batches:
+// gather, BWT (shared memory up to BZ_SMEM_MAX_N bytes, else global scratch), MTF + table choice + bit count.  Device
+// memory of a batch is bounded by BZ_BATCH_BYTES whatever the number of jobs.
+constexpr uint64_t BZ_BATCH_BYTES = 192ull << 20;
+constexpr size_t BZ_BATCH_BLOCKS = 1 << 16;
+
+// RLE1 of every sequence, its emission-start flags (a host copy plans the block cuts), where the open block of each
+// sequence alone starts, and the bits of its closed blocks once computed
+struct BzState {
+    bool ready = false;
+    DevBuf rle, flag;
+    BzSeq *d_info = nullptr;
+    unsigned long long *d_seq_bits = nullptr;
+    std::vector<BzSeq> h_info; std::vector<uint8_t> h_flag, h_pdone;
+    std::vector<uint32_t> h_open, h_nclosed;
+    // working memory: argument arrays and batch buffers
+    DevBuf all, blocks, small, large, buf, bwt, mtf, job_bits, job_prefix;
+    cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+    // options "bzip2_smem", "bzip2_prefix" (0: for tests, same results)
+    int use_smem = 1, use_prefix = 1;
+    // statistics of the last call
+    int64_t n_blocks = 0, smem_blocks = 0, prefix_blocks = 0;
+    double ms[4] = {0, 0, 0, 0};               // RLE1 + gather, BWT small, BWT large, MTF + selection + bits
+};
+
+static inline void bz_free_corpus(BzState &st)
+{
+    st.rle.release(); st.flag.release();
+    cudaFree(st.d_info); st.d_info = nullptr;
+    cudaFree(st.d_seq_bits); st.d_seq_bits = nullptr;
+    st.ready = false;
+}
+
+static inline void bz_free_work(BzState &st)
+{
+    for (DevBuf *b : {&st.all, &st.blocks, &st.small, &st.large, &st.buf, &st.bwt, &st.mtf, &st.job_bits, &st.job_prefix})
+        b->release();
+    for (cudaEvent_t &e : st.ev) { if (e) cudaEventDestroy(e); e = nullptr; }
+}
+
+// the RLE1 of the corpus is computed again by the next call
+static inline void bz_invalidate(BzState &st) { st.ready = false; }
+
+static int bz_prepare(BzState &st, const Corpus &c, cudaStream_t stream, int64_t *launches, std::string &err)
+{
+    NvtxRange nvtx_("snacc_b200: bzip2 RLE1");
+    const int32_t n = c.n_seqs;
+    st.h_info.assign((size_t)n, BzSeq{});
+    uint64_t cap = 0;
+    for (int32_t i = 0; i < n; ++i) { st.h_info[i].roff = cap; cap += (uint64_t)c.h_len[i] / 4 * 5 + 16; }
+    DCK(st.rle.grow(cap, stream, true));
+    DCK(st.flag.grow(cap, stream, true));
+    if (!st.d_info) DCK(cudaMalloc(&st.d_info, sizeof(BzSeq) * n));
+    if (!st.d_seq_bits) DCK(cudaMalloc(&st.d_seq_bits, sizeof(unsigned long long) * n));
+    DCK(cudaMemsetAsync(st.d_seq_bits, 0, sizeof(unsigned long long) * n, stream));
+    DCK(cudaMemcpyAsync(st.d_info, st.h_info.data(), sizeof(BzSeq) * n, cudaMemcpyHostToDevice, stream));
+    std::vector<int32_t> all((size_t)n);
+    for (int32_t i = 0; i < n; ++i) all[i] = i;
+    DCK(st.all.grow(sizeof(int32_t) * n, stream));
+    DCK(cudaMemcpyAsync(st.all.p, all.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice, stream));
+    bz_rle_kernel<<<(n + 31) / 32, 32, 0, stream>>>(c.d_corpus, c.d_off, c.d_len, st.all.get<int32_t>(), n,
+                                                    st.rle.get<uint8_t>(), st.flag.get<uint8_t>(), st.d_info);
+    DCK(cudaGetLastError());
+    ++*launches;
+    st.h_flag.resize(cap);
+    DCK(cudaMemcpyAsync(st.h_info.data(), st.d_info, sizeof(BzSeq) * n, cudaMemcpyDeviceToHost, stream));
+    DCK(cudaMemcpyAsync(st.h_flag.data(), st.flag.p, cap, cudaMemcpyDeviceToHost, stream));
+    DCK(cudaStreamSynchronize(stream));
+    // where the last block of each sequence alone starts: the blocks before it close the same way in every x.y
+    st.h_open.assign((size_t)n, 0); st.h_nclosed.assign((size_t)n, 0); st.h_pdone.assign((size_t)n, 0);
+    std::vector<BzWin> wins;
+    for (int32_t i = 0; i < n; ++i) {
+        const BzSeq &si = st.h_info[i];
+        if (si.rlen <= BZ_NBLOCK_MAX) continue;
+        const uint8_t *f = st.h_flag.data() + si.roff;
+        wins.clear();
+        bz_cut(bz_view_single(0, si.rlen), f, f, wins);
+        st.h_open[i] = wins.back().v0;
+        st.h_nclosed[i] = (uint32_t)wins.size() - 1;
+    }
+    st.ready = true;
+    return 0;
+}
+
+// one batch of blocks; `work` holds the global-memory sort's 4 arrays of 32-bit words per block byte
+static int bz_run_batch(BzState &st, const BzBlock *blocks, size_t nb, uint64_t bytes, unsigned long long *d_job_bits,
+                        DevBuf &work, cudaStream_t stream, int64_t *launches, std::string &err)
+{
+    NvtxRange nvtx_("snacc_b200: bzip2 batch");
+    std::vector<int32_t> small, large;
+    for (size_t k = 0; k < nb; ++k)
+        ((st.use_smem && blocks[k].n <= BZ_SMEM_MAX_N) ? small : large).push_back((int32_t)k);
+    DCK(st.blocks.grow(sizeof(BzBlock) * nb, stream));
+    DCK(st.small.grow(sizeof(int32_t) * (small.size() + 1), stream));
+    DCK(st.large.grow(sizeof(int32_t) * (large.size() + 1), stream));
+    DCK(st.buf.grow(bytes, stream));
+    DCK(st.bwt.grow(bytes, stream));
+    DCK(st.mtf.grow(sizeof(uint16_t) * (bytes + nb), stream));
+    if (!large.empty()) DCK(work.grow(16 * bytes, stream, true));
+    const BzBlock *d_blocks = st.blocks.get<BzBlock>();
+    const int32_t *d_small = st.small.get<int32_t>(), *d_large = st.large.get<int32_t>();
+    uint8_t *d_buf = st.buf.get<uint8_t>(), *d_bwt = st.bwt.get<uint8_t>();
+    DCK(cudaMemcpyAsync(st.blocks.p, blocks, sizeof(BzBlock) * nb, cudaMemcpyHostToDevice, stream));
+    if (!small.empty()) DCK(cudaMemcpyAsync(st.small.p, small.data(), sizeof(int32_t) * small.size(), cudaMemcpyHostToDevice, stream));
+    if (!large.empty()) DCK(cudaMemcpyAsync(st.large.p, large.data(), sizeof(int32_t) * large.size(), cudaMemcpyHostToDevice, stream));
+    DCK(cudaEventRecord(st.ev[0], stream));
+    bz_gather_kernel<<<(unsigned)nb, 256, 0, stream>>>(d_blocks, st.d_info, st.rle.get<uint8_t>(), st.flag.get<uint8_t>(), d_buf);
+    DCK(cudaGetLastError());
+    DCK(cudaEventRecord(st.ev[1], stream));
+    if (!small.empty()) {
+        DCK(cudaFuncSetAttribute(bz_bwt_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BZ_SMEM_BYTES));
+        bz_bwt_smem_kernel<<<(unsigned)small.size(), BZ_SORT_THREADS, BZ_SMEM_BYTES, stream>>>(d_blocks, d_small, d_buf, d_bwt);
+        DCK(cudaGetLastError());
+    }
+    DCK(cudaEventRecord(st.ev[2], stream));
+    if (!large.empty()) {
+        bz_bwt_global_kernel<<<(unsigned)large.size(), BZ_SORT_THREADS, 0, stream>>>(d_blocks, d_large, d_buf, d_bwt,
+                                                                                      work.get<uint32_t>());
+        DCK(cudaGetLastError());
+    }
+    DCK(cudaEventRecord(st.ev[3], stream));
+    DCK(cudaFuncSetAttribute(bz_bits_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BZ_BITS_DYN_SMEM));
+    bz_bits_kernel<<<(unsigned)nb, BZ_BITS_THREADS, BZ_BITS_DYN_SMEM, stream>>>(d_blocks, d_bwt, st.mtf.get<uint16_t>(),
+                                                                               d_job_bits, st.d_seq_bits);
+    DCK(cudaGetLastError());
+    DCK(cudaEventRecord(st.ev[4], stream));
+    DCK(cudaEventSynchronize(st.ev[4]));
+    for (int s = 0; s < 4; ++s) {
+        float ms = 0.f;
+        DCK(cudaEventElapsedTime(&ms, st.ev[s], st.ev[s + 1]));
+        st.ms[s] += ms;
+    }
+    *launches += 2 + !small.empty() + !large.empty();
+    st.n_blocks += (int64_t)nb;
+    st.smem_blocks += (int64_t)small.size();
+    return 0;
+}
+
+// A job list (ys null: singles) into d_out.  d_xs: the x list on the device.
+static int bz_run(BzState &st, const Corpus &c, const int32_t *xs, const int32_t *ys, const int32_t *d_xs,
+                  int64_t n_jobs, int64_t *d_out, DevBuf &work, cudaStream_t stream, int64_t *launches, std::string &err)
+{
+    st.n_blocks = st.smem_blocks = st.prefix_blocks = 0;
+    for (double &m : st.ms) m = 0;
+    for (cudaEvent_t &e : st.ev) if (!e) DCK(cudaEventCreate(&e));
+    if (!st.ready) {
+        DCK(cudaEventRecord(st.ev[0], stream));
+        int r = bz_prepare(st, c, stream, launches, err);
+        if (r) return r;
+        DCK(cudaEventRecord(st.ev[1], stream));
+        DCK(cudaEventSynchronize(st.ev[1]));
+        float ms = 0.f;
+        DCK(cudaEventElapsedTime(&ms, st.ev[0], st.ev[1]));
+        st.ms[0] += ms;
+    }
+    DCK(st.job_bits.grow(sizeof(unsigned long long) * n_jobs, stream));
+    DCK(st.job_prefix.grow((size_t)n_jobs, stream));
+    unsigned long long *d_job_bits = st.job_bits.get<unsigned long long>();
+    DCK(cudaMemsetAsync(d_job_bits, 0, sizeof(unsigned long long) * n_jobs, stream));
+    std::vector<uint8_t> use_prefix((size_t)n_jobs, 0);
+    std::vector<BzBlock> batch;
+    batch.reserve(BZ_BATCH_BLOCKS);
+    uint64_t bytes = 0;
+    std::vector<BzWin> wins;
+    const uint8_t *hf = st.h_flag.data();
+    int64_t computed_closed = 0, used_closed = 0;
+    // blocks of the view v of job/sequence `dst` go into the batch, which runs whenever it is full
+    auto add = [&](int64_t dst, int32_t x, int32_t y, const BzView &v) -> int {
+        const BzSeq &sx = st.h_info[x], &sy = st.h_info[y < 0 ? x : y];
+        wins.clear();
+        bz_cut(v, hf + sx.roff, hf + sy.roff, wins);
+        for (const BzWin &w : wins) {
+            if (batch.size() == BZ_BATCH_BLOCKS || bytes + w.n > BZ_BATCH_BYTES) {
+                int r = bz_run_batch(st, batch.data(), batch.size(), bytes, d_job_bits, work, stream, launches, err);
+                if (r) return r;
+                batch.clear(); bytes = 0;
+            }
+            batch.push_back(BzBlock{dst, bytes, x, y, w.v0, w.n, v});
+            bytes += (w.n + 15) & ~15u;
+        }
+        return 0;
+    };
+    for (int64_t k = 0; k < n_jobs; ++k) {
+        const int32_t x = xs[k], y = ys ? ys[k] : -1;
+        const uint32_t open = st.h_open[x];
+        int r;
+        if (open) {
+            if (st.use_prefix) {
+                use_prefix[k] = 1;
+                used_closed += st.h_nclosed[x];
+                if (!st.h_pdone[x]) {
+                    st.h_pdone[x] = 1;
+                    computed_closed += st.h_nclosed[x];
+                    if ((r = add(-1 - (int64_t)x, x, -1, bz_view_single(0, open)))) return r;
+                }
+            } else if ((r = add(k, x, -1, bz_view_single(0, open)))) return r;
+        }
+        const BzSeq &sx = st.h_info[x];
+        if ((r = add(k, x, y, y < 0 ? bz_view_single(open, sx.rlen) : bz_view_pair(sx, open, st.h_info[y])))) return r;
+    }
+    if (!batch.empty()) {
+        const int r = bz_run_batch(st, batch.data(), batch.size(), bytes, d_job_bits, work, stream, launches, err);
+        if (r) return r;
+    }
+    st.prefix_blocks = used_closed - computed_closed;
+    DCK(cudaMemcpyAsync(st.job_prefix.p, use_prefix.data(), (size_t)n_jobs, cudaMemcpyHostToDevice, stream));
+    const int blocks = (int)std::min<int64_t>((n_jobs + 255) / 256, 148 * 8);
+    bz_finish_kernel<<<blocks, 256, 0, stream>>>(d_job_bits, st.d_seq_bits, d_xs, st.job_prefix.get<uint8_t>(), n_jobs, d_out);
+    DCK(cudaGetLastError());
+    ++*launches;
+    return 0;
 }
 
 #endif  // __CUDACC__

@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdio.h>
 
 // Device code is also compilable for the host so that tests/host_emu.cu can run the very same parse
 // functions on the CPU against the oracle (test infrastructure; the product never does this).
@@ -77,5 +78,44 @@ SNACC_HD uint8_t ld8(const Stream &s, uint32_t p)
 {
     return p >= s.lx ? SNACC_LDG(s.y + (p - s.lx)) : SNACC_LDG(s.x + p);
 }
+
+#ifdef __CUDACC__
+// ---- host side of the codec drivers ----------------------------------------------------------------------------------
+
+// the uploaded corpus as the codec drivers see it (device arrays and their host copies)
+struct Corpus {
+    const uint8_t *d_corpus; const uint64_t *d_off; const uint32_t *d_len;
+    const uint64_t *h_off; const uint32_t *h_len; int32_t n_seqs;
+};
+
+// A device array that grows on demand and is kept between calls (all its use is ordered on one stream).  Growing
+// synchronises the stream first: an earlier launch may still read the old array.  Small argument arrays get 1.25x
+// headroom (4 KiB at least) so that calls of slowly growing size do not reallocate every time; the large ones (job
+// arrays, outputs, working tables) are sized exactly, since headroom there would be memory held between calls for nothing.
+struct DevBuf {
+    void *p = nullptr;
+    size_t cap = 0;
+    template <typename T> T *get() const { return (T *)p; }
+    cudaError_t grow(size_t bytes, cudaStream_t stream, bool exact = false)
+    {
+        if (bytes <= cap) return cudaSuccess;
+        cudaError_t e = cudaStreamSynchronize(stream);
+        if (e != cudaSuccess) return e;
+        release();
+        const size_t want = exact ? bytes : (bytes + bytes / 4 > 4096 ? bytes + bytes / 4 : 4096);
+        e = cudaMalloc(&p, want);
+        if (e != cudaSuccess) { p = nullptr; return e; }
+        cap = want;
+        return cudaSuccess;
+    }
+    void release() { cudaFree(p); p = nullptr; cap = 0; }
+};
+
+// codec drivers: a failed CUDA call records its message in `err` (a std::string in scope) and the function returns
+// SNACC_ERR_CUDA (-1)
+#define DCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { \
+        char b_[512]; snprintf(b_, sizeof b_, "%s failed at %s:%d: %s", #call, __FILE__, __LINE__, cudaGetErrorString(e_)); \
+        err = b_; return -1; } } while (0)
+#endif  // __CUDACC__
 
 }  // namespace snacc

@@ -2043,11 +2043,6 @@ __global__ void dfl_gather_sizes_kernel(const int64_t *__restrict__ seq_size, co
 // ------------------------------------------------------------------------------------------------
 // host-side orchestration (called from api.cu with the context lock held)
 // ------------------------------------------------------------------------------------------------
-struct DeflateCorpus {
-    const uint8_t *d_corpus; const uint64_t *d_off; const uint32_t *d_len;
-    const uint64_t *h_off; const uint32_t *h_len; int32_t n_seqs;
-};
-
 // Device state of the deflate codecs, split by the role a sequence plays (DflCorpus):
 //   x side, every sequence: its record (checkpoint + size alone), its tail 3-byte index (the whole index with
 //     deflate_tail_index 0), tail counts and tail 6-byte pack -- what a pair stream x.* needs of x;
@@ -2219,10 +2214,6 @@ static inline void deflate_invalidate(DeflateState &st)
     }
 }
 
-#define DCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { \
-        char b_[512]; snprintf(b_, sizeof b_, "%s failed at %s:%d: %s", #call, __FILE__, __LINE__, cudaGetErrorString(e_)); \
-        err = b_; return -1; } } while (0)
-
 template <typename T> static int dfl_upload(std::string &err, cudaStream_t stream, const std::vector<T> &h, T **d)
 {
     *d = nullptr;
@@ -2281,7 +2272,7 @@ static int dfl_build_index(DeflateState &st, const DflCorpus &c, const std::vect
 }
 
 // x side of every sequence (allocated on first use, and again when the x index layout changes)
-static int deflate_ensure_x(DeflateState &st, const DeflateCorpus &dc, int level, cudaStream_t stream, std::string &err)
+static int deflate_ensure_x(DeflateState &st, const Corpus &dc, int level, cudaStream_t stream, std::string &err)
 {
     const int li = level == 9 ? 0 : 1;
     const int32_t ns = dc.n_seqs;
@@ -2352,7 +2343,7 @@ static int deflate_ensure_y_level(DeflateState &st, int level, std::string &err)
     return 0;
 }
 
-static int deflate_layout_arrays(DeflateState &st, const DeflateCorpus &dc, int level, const std::vector<int32_t> &list,
+static int deflate_layout_arrays(DeflateState &st, const Corpus &dc, int level, const std::vector<int32_t> &list,
                                  cudaStream_t stream, std::string &err)
 {
     deflate_drop_y(st);
@@ -2381,7 +2372,7 @@ static int deflate_layout_arrays(DeflateState &st, const DeflateCorpus &dc, int 
     return deflate_alloc_y_level(st, level, err);
 }
 // a new y layout holding exactly `list` (ascending): the previous one is dropped; on failure there is no layout
-static int deflate_set_layout(DeflateState &st, const DeflateCorpus &dc, int level, const std::vector<int32_t> &list,
+static int deflate_set_layout(DeflateState &st, const Corpus &dc, int level, const std::vector<int32_t> &list,
                               cudaStream_t stream, std::string &err)
 {
     if (deflate_layout_arrays(st, dc, level, list, stream, err)) { deflate_drop_y(st); return -1; }
@@ -2399,7 +2390,7 @@ static int deflate_upload_ix(DeflateState &st, cudaStream_t stream, std::string 
     return 0;
 }
 
-static DflCorpus deflate_corpus(const DeflateState &st, const DeflateCorpus &dc, int li)
+static DflCorpus deflate_corpus(const DeflateState &st, const Corpus &dc, int li)
 {
     return DflCorpus{dc.d_corpus, dc.d_off, dc.d_len, st.d_poff, st.d_ix, st.d_yslot, st.d_yindex,
                      st.d_head_order, st.d_head_visit[li],
@@ -2427,7 +2418,7 @@ static int dfl_index_packs(const DflCorpus &c, const std::vector<int32_t> &list,
 
 // x index slices of the listed sequences (their last DFL_XTAIL positions, or whole with deflate_tail_index 0): the
 // junction walks of a pair stream x.y reach at most 264 + 32 768 positions back from the end of x
-static int deflate_build_x(DeflateState &st, const DeflateCorpus &dc, int li, const std::vector<int32_t> &list,
+static int deflate_build_x(DeflateState &st, const Corpus &dc, int li, const std::vector<int32_t> &list,
                            cudaStream_t stream, int64_t *launches, std::string &err)
 {
     if (list.empty()) return 0;
@@ -2459,7 +2450,7 @@ static int deflate_build_x(DeflateState &st, const DeflateCorpus &dc, int li, co
 
 // the full preparation of the listed sequences of the y layout that lack it: whole index, F of this level and the
 // parse of the sequence alone (size, checkpoint, canonical symbol stream)
-static int deflate_prepare_y(DeflateState &st, const DeflateCorpus &dc, int level, const std::vector<int32_t> &list,
+static int deflate_prepare_y(DeflateState &st, const Corpus &dc, int level, const std::vector<int32_t> &list,
                              cudaStream_t stream, int64_t *launches, std::string &err)
 {
     const int li = level == 9 ? 0 : 1;
@@ -2623,7 +2614,7 @@ static int deflate_prepare_y(DeflateState &st, const DeflateCorpus &dc, int leve
 // them (sharding.py: each rank parses its own band of sequences, one all-gather of these records).
 struct DflPrefixRecord { DflCkpt ck; int64_t size; };
 
-static int deflate_export_prefix(DeflateState &st, const DeflateCorpus &dc, int level, const int32_t *seqs, int64_t n,
+static int deflate_export_prefix(DeflateState &st, const Corpus &dc, int level, const int32_t *seqs, int64_t n,
                                  DflPrefixRecord *out, cudaStream_t stream, std::string &err)
 {
     const int li = level == 9 ? 0 : 1;
@@ -2638,7 +2629,7 @@ static int deflate_export_prefix(DeflateState &st, const DeflateCorpus &dc, int 
     return 0;
 }
 
-static int deflate_import_prefix(DeflateState &st, const DeflateCorpus &dc, int level, const int32_t *seqs, int64_t n,
+static int deflate_import_prefix(DeflateState &st, const Corpus &dc, int level, const int32_t *seqs, int64_t n,
                                  const DflPrefixRecord *in, cudaStream_t stream, std::string &err)
 {
     const int li = level == 9 ? 0 : 1;
@@ -2656,7 +2647,7 @@ static int deflate_import_prefix(DeflateState &st, const DeflateCorpus &dc, int 
 }
 
 // pair jobs (all, or the listed subset) through the junction / parse batches; sizes land at d_out[job]
-static int deflate_pairs(DeflateState &st, const DeflateCorpus &dc, int level, const int32_t *xs, const int32_t *ys,
+static int deflate_pairs(DeflateState &st, const Corpus &dc, int level, const int32_t *xs, const int32_t *ys,
                          int64_t n_jobs, const std::vector<int64_t> *subset, int kind, size_t batch, int64_t *d_out,
                          cudaStream_t stream, int64_t *launches, std::string &err)
 {
@@ -2763,9 +2754,9 @@ static int deflate_pairs(DeflateState &st, const DeflateCorpus &dc, int level, c
 }
 
 // sizes of the raw deflate streams of the jobs (x alone when ys == nullptr) into d_out[0..n_jobs)
-static int deflate_run(DeflateState &st, const DeflateCorpus &dc, int level, const int32_t *xs, const int32_t *ys,
-                       const int32_t *d_xs, const int32_t *, int64_t n_jobs, int64_t *d_out, cudaStream_t stream,
-                       int64_t, int64_t *launches, std::string &err)
+static int deflate_run(DeflateState &st, const Corpus &dc, int level, const int32_t *xs, const int32_t *ys,
+                       const int32_t *d_xs, int64_t n_jobs, int64_t *d_out, cudaStream_t stream, int64_t *launches,
+                       std::string &err)
 {
     const int li = level == 9 ? 0 : 1;
     const int32_t ns = dc.n_seqs;
@@ -2928,7 +2919,6 @@ static int deflate_run(DeflateState &st, const DeflateCorpus &dc, int level, con
     }
     return 0;
 }
-#undef DCK
 #endif  // __CUDACC__
 
 }  // namespace snacc
