@@ -127,7 +127,10 @@ int snacc_ncd(snacc_ctx *ctx, const int64_t *C, const int64_t *S, int32_t n, int
 
 /* Downstream of the matrix (SURVEY.md 8f rank 4): metrify -- 0.5 (D + D^T), zero diagonal, snacc/misc.py:20-25 -- when
  * `metrify` is non-zero, then UPGMA, i.e. scipy.cluster.hierarchy.linkage(squareform(D_sym), method='average') of
- * snacc/distmatrix_to_tree.py:9-15.  Z receives scipy's linkage matrix, (n-1) rows of (id_a < id_b, height, leaves). */
+ * snacc/distmatrix_to_tree.py:9-15.  Z receives scipy's linkage matrix, (n-1) rows of (id_a < id_b, height, leaves),
+ * bit for bit, ties included (scipy's nearest-neighbour chain, stable sort by height and relabelling).  Returns
+ * SNACC_ERR_ARG, with a message, for input scipy rejects: n < 2, a non-finite entry in the matrix to be clustered
+ * (after metrify), and with `metrify` == 0 an asymmetric matrix or a non-zero diagonal. */
 int snacc_upgma(snacc_ctx *ctx, const double *D, int32_t n, int metrify, double *Z);
 
 /* ---- instrumentation used by bench.py ---- */

@@ -648,6 +648,28 @@ extern "C" int snacc_ncd(snacc_ctx *ctx, const int64_t *C, const int64_t *S, int
     return SNACC_OK;
 }
 
+// scipy's label(): the merges, sorted by height, name their clusters by slot; a union-find over the leaves turns each
+// slot into the id of the cluster that holds it (n, n+1, ... in row order), smaller id first
+static void upgma_label(double *Z, int32_t n)
+{
+    std::vector<int32_t> parent(2 * (size_t)n - 1), count(2 * (size_t)n - 1, 1);
+    for (int32_t i = 0; i < 2 * n - 1; ++i) parent[i] = i;
+    auto find = [&](int32_t a) {
+        int32_t r = a;
+        while (parent[r] != r) r = parent[r];
+        while (parent[a] != r) { const int32_t p = parent[a]; parent[a] = r; a = p; }
+        return r;
+    };
+    for (int32_t k = 0; k + 1 < n; ++k) {
+        const int32_t a = find((int32_t)Z[4 * (size_t)k]), b = find((int32_t)Z[4 * (size_t)k + 1]);
+        Z[4 * (size_t)k + 0] = (double)std::min(a, b);
+        Z[4 * (size_t)k + 1] = (double)std::max(a, b);
+        parent[a] = parent[b] = n + k;
+        count[n + k] = count[a] + count[b];
+        Z[4 * (size_t)k + 3] = (double)count[n + k];
+    }
+}
+
 // downstream of the distance matrix: metrify (misc.py:20-25) + UPGMA (distmatrix_to_tree.py:9-15) -> scipy's linkage matrix
 extern "C" int snacc_upgma(snacc_ctx *ctx, const double *D, int32_t n, int metrify, double *Z)
 {
@@ -658,33 +680,55 @@ extern "C" int snacc_upgma(snacc_ctx *ctx, const double *D, int32_t n, int metri
     NvtxRange nvtx_("snacc_b200: metrify + upgma");
     CK(cudaSetDevice(ctx->device));
     const size_t nn = (size_t)n * n;
-    double *dD = nullptr, *dM = nullptr, *dZ = nullptr, *d_nnv = nullptr;
-    int32_t *d_size = nullptr, *d_label = nullptr, *d_nni = nullptr, *d_todo = nullptr;
-    uint8_t *d_active = nullptr;
+    double *dD = nullptr, *dM = nullptr, *dZ = nullptr;
+    int32_t *d_size = nullptr, *d_chain = nullptr;
+    int *d_flags = nullptr;
     auto release = [&]() {
-        cudaFree(dD); cudaFree(dM); cudaFree(dZ); cudaFree(d_nnv); cudaFree(d_size); cudaFree(d_label); cudaFree(d_nni);
-        cudaFree(d_todo); cudaFree(d_active);
+        cudaFree(dD); cudaFree(dM); cudaFree(dZ); cudaFree(d_size); cudaFree(d_chain); cudaFree(d_flags);
     };
 #define UCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { release(); \
         ctx->err = std::string(#call " failed: ") + cudaGetErrorString(e_); return SNACC_ERR_CUDA; } } while (0)
     UCK(cudaMalloc(&dD, sizeof(double) * nn));
     UCK(cudaMalloc(&dM, sizeof(double) * nn));
     UCK(cudaMalloc(&dZ, sizeof(double) * 4 * (size_t)(n - 1)));
-    UCK(cudaMalloc(&d_nnv, sizeof(double) * n));
     UCK(cudaMalloc(&d_size, sizeof(int32_t) * n));
-    UCK(cudaMalloc(&d_label, sizeof(int32_t) * n));
-    UCK(cudaMalloc(&d_nni, sizeof(int32_t) * n));
-    UCK(cudaMalloc(&d_todo, sizeof(int32_t) * (n + 1)));
-    UCK(cudaMalloc(&d_active, (size_t)n));
+    UCK(cudaMalloc(&d_chain, sizeof(int32_t) * n));
+    UCK(cudaMalloc(&d_flags, sizeof(int)));
     UCK(cudaMemcpyAsync(dD, D, sizeof(double) * nn, cudaMemcpyHostToDevice, ctx->stream));
-    metrify_kernel<<<(unsigned)std::min<size_t>((nn + 255) / 256, 148 * 8), 256, 0, ctx->stream>>>(dD, n, metrify ? 1 : 0, dM);
+    UCK(cudaMemsetAsync(d_flags, 0, sizeof(int), ctx->stream));
+    const unsigned grid = (unsigned)std::min<size_t>((nn + 255) / 256, 148 * 8);
+    metrify_kernel<<<grid, 256, 0, ctx->stream>>>(dD, n, metrify ? 1 : 0, dM);
     UCK(cudaGetLastError());
-    upgma_kernel<<<1, UPGMA_THREADS, 0, ctx->stream>>>(dM, n, dZ, d_size, d_label, d_nni, d_nnv, d_active, d_todo);
+    // what scipy's squareform and linkage refuse: checked on the matrix to be clustered, before the UPGMA launch
+    upgma_check_kernel<<<grid, 256, 0, ctx->stream>>>(dM, n, metrify ? 0 : 1, d_flags);
+    UCK(cudaGetLastError());
+    int flags = 0;
+    UCK(cudaMemcpyAsync(&flags, d_flags, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    UCK(cudaStreamSynchronize(ctx->stream));
+    if (flags) {
+        release();
+        std::string msg = "snacc_upgma: the distance matrix";
+        if (flags & UPGMA_NONFINITE) msg += " must contain only finite values;";
+        if (flags & UPGMA_ASYMMETRIC) msg += " must be symmetric;";
+        if (flags & UPGMA_DIAGONAL) msg += " must have a zero diagonal;";
+        msg.back() = ' ';
+        msg += metrify ? "(after metrify)" : "(metrify is off)";
+        FAIL(SNACC_ERR_ARG, msg);
+    }
+    upgma_kernel<<<1, UPGMA_THREADS, 0, ctx->stream>>>(dM, n, dZ, d_size, d_chain);
     UCK(cudaGetLastError());
     UCK(cudaMemcpyAsync(Z, dZ, sizeof(double) * 4 * (size_t)(n - 1), cudaMemcpyDeviceToHost, ctx->stream));
     UCK(cudaStreamSynchronize(ctx->stream));
 #undef UCK
     release();
+    // the rows come in merge order with slot ids: sort them stably by height (numpy's mergesort), then scipy's labels
+    std::vector<double> raw(Z, Z + 4 * (size_t)(n - 1));
+    std::vector<int32_t> order(n - 1);
+    for (int32_t k = 0; k + 1 < n; ++k) order[k] = k;
+    std::stable_sort(order.begin(), order.end(), [&](int32_t a, int32_t b) { return raw[4 * (size_t)a + 2] < raw[4 * (size_t)b + 2]; });
+    for (int32_t k = 0; k + 1 < n; ++k)
+        for (int c = 0; c < 4; ++c) Z[4 * (size_t)k + c] = raw[4 * (size_t)order[k] + c];
+    upgma_label(Z, n);
     return SNACC_OK;
 }
 

@@ -1,16 +1,23 @@
 // upgma.cuh -- K5: the downstream step of the distance matrix on the device (SURVEY.md 8f rank 4), sm_100a.
 //   metrify      snacc/misc.py:20-25               D_sym = 0.5 (D + D^T), zero diagonal
 //   hierarchical snacc/distmatrix_to_tree.py:9-15  scipy.cluster.hierarchy.linkage(squareform(D_sym), method='average')
-// Output is scipy's linkage matrix Z ((n-1) x 4: cluster ids a < b, height, leaf count; new clusters are numbered n, n+1,
-// ... in merge order).  UPGMA is a reducible linkage, so merging the globally closest pair each step gives the same
-// hierarchy, in the same (non-decreasing height) order scipy sorts its nearest-neighbour-chain result into; heights use
-// the same update d(k, a+b) = (|a| d(k,a) + |b| d(k,b)) / (|a| + |b|).  (Exactly tied heights may be ordered
-// differently; real NCD matrices have none.)
+// Output is scipy's linkage matrix Z ((n-1) x 4: cluster ids a < b, height, leaf count; new clusters are numbered n,
+// n+1, ... in row order), bit for bit, ties included.  An NCD is a ratio of integer sizes, so real matrices have many
+// equal distances, and with ties the order of the merges decides the tree.  So the kernel runs scipy's own algorithm,
+// nn_chain (scipy/cluster/_hierarchy.pyx), not some other reducible-linkage order:
+//   * the chain starts at the first active slot; each step takes the closest active cluster y of the chain's top x
+//     (ties: smallest slot), and takes it only when it is strictly closer than the previous chain element;
+//   * when the step returns the previous element, x and y merge: with x < y, the merged cluster goes to slot y and
+//     slot x is dropped; the row (x, y, height, size) is recorded in merge order;
+//   * the update is d(i, y) = (|x| d(i, x) + |y| d(i, y)) / (|x| + |y|) with every product and sum rounded on its own
+//     (__dmul_rn / __dadd_rn / __ddiv_rn: a fused multiply-add would change the last bit of a height).
+// The host (snacc_upgma) then sorts the rows stably by height and relabels them with a union-find, as scipy's
+// label() does.  Input scipy rejects (non-finite values; with metrify off, an asymmetric matrix or a non-zero
+// diagonal) is found by upgma_check_kernel and refused before upgma_kernel is launched.
 //
-// One CTA walks the n-1 merges (the chain of merges is serial); all the work inside a step is parallel over its 1024
-// threads: a nearest-neighbour entry per row (closest active column to its right) makes the global minimum an O(n)
-// reduction and the update O(n) plus the rescans of the few rows whose neighbour was merged away.  The matrix stays in
-// HBM / L2 (n = 10 000: 800 MB); nothing here is a dense contraction.
+// One CTA walks the chain (the steps are serial); each step is one parallel argmin over row x, a contiguous read of n
+// doubles, and each merge one parallel update of row and column y.  The matrix stays in HBM / L2 (n = 10 000:
+// 800 MB); nothing here is a dense contraction.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -26,93 +33,98 @@ __global__ void metrify_kernel(const double *__restrict__ D, int32_t n, int do_m
     }
 }
 
-constexpr int UPGMA_THREADS = 1024;
+// what scipy refuses in the matrix to be clustered, OR-ed into *flags
+constexpr int UPGMA_NONFINITE = 1, UPGMA_ASYMMETRIC = 2, UPGMA_DIAGONAL = 4;
 
-// closest active column j > k of row k (ties: smallest j), by one warp
-__device__ __forceinline__ void upgma_rescan(const double *M, int32_t n, const uint8_t *active, int32_t k, int32_t lane,
-                                             double *nn_val, int32_t *nn_idx)
+__global__ void upgma_check_kernel(const double *__restrict__ M, int32_t n, int check_square_form, int *__restrict__ flags)
 {
-    double bv = 1.0 / 0.0;
-    int32_t bj = -1;
-    for (int32_t j = k + 1 + lane; j < n; j += 32) {
-        if (!active[j]) continue;
-        const double v = M[(int64_t)k * n + j];
-        if (v < bv) { bv = v; bj = j; }
+    const int64_t total = (int64_t)n * n;
+    int f = 0;
+    for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < total; k += (int64_t)gridDim.x * blockDim.x) {
+        const int32_t i = (int32_t)(k / n), j = (int32_t)(k % n);
+        const double v = M[k];
+        if (i != j && !isfinite(v)) f |= UPGMA_NONFINITE;
+        if (check_square_form) {
+            if (i == j && v != 0.0) f |= UPGMA_DIAGONAL;
+            if (i < j && !(v == M[(int64_t)j * n + i])) f |= UPGMA_ASYMMETRIC;
+        }
     }
-    for (int off = 16; off; off >>= 1) {
-        const double ov = __shfl_down_sync(0xffffffffu, bv, off);
-        const int32_t oj = __shfl_down_sync(0xffffffffu, bj, off);
-        if (oj >= 0 && (bj < 0 || ov < bv || (ov == bv && oj < bj))) { bv = ov; bj = oj; }
-    }
-    if (lane == 0) { nn_val[k] = bv; nn_idx[k] = bj; }
+    if (f) atomicOr(flags, f);
 }
 
+constexpr int UPGMA_THREADS = 1024;
+
+// the smaller of two (value, slot) candidates; ties: smaller slot
+__device__ __forceinline__ void upgma_take_min(double &bv, int32_t &bi, double ov, int32_t oi)
+{
+    if (ov < bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+}
+
+// M: the symmetric n x n matrix, overwritten.  Z: the (n-1) x 4 merges in merge order, with slot ids (x < y) -- the
+// host sorts and relabels them.  size: n ints (0 = dropped slot).  chain: n ints.
 __global__ void __launch_bounds__(UPGMA_THREADS)
-upgma_kernel(double *__restrict__ M, int32_t n, double *__restrict__ Z, int32_t *__restrict__ size, int32_t *__restrict__ label,
-             int32_t *__restrict__ nn_idx, double *__restrict__ nn_val, uint8_t *__restrict__ active, int32_t *__restrict__ todo)
+upgma_kernel(double *__restrict__ M, int32_t n, double *__restrict__ Z, int32_t *__restrict__ size, int32_t *__restrict__ chain)
 {
     __shared__ double s_val[UPGMA_THREADS / 32];
-    __shared__ int32_t s_row[UPGMA_THREADS / 32];
-    __shared__ int32_t s_a, s_b, s_ntodo;
-    const int32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarp = UPGMA_THREADS / 32;
-    for (int32_t i = tid; i < n; i += UPGMA_THREADS) { size[i] = 1; label[i] = i; active[i] = 1; }
+    __shared__ int32_t s_idx[UPGMA_THREADS / 32];
+    __shared__ int32_t s_x, s_y, s_len, s_first, s_merge;
+    const int32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    for (int32_t i = tid; i < n; i += UPGMA_THREADS) size[i] = 1;
+    if (tid == 0) { s_len = 0; s_first = 0; }
     __syncthreads();
-    for (int32_t k = warp; k < n; k += nwarp) upgma_rescan(M, n, active, k, lane, nn_val, nn_idx);
-    __syncthreads();
-    for (int32_t t = 0; t + 1 < n; ++t) {
-        // (1) the closest pair: minimum over the rows' nearest neighbours (ties: smallest row)
-        double bv = 1.0 / 0.0;
-        int32_t bi = -1;
-        for (int32_t i = tid; i < n; i += UPGMA_THREADS) {
-            if (!active[i] || nn_idx[i] < 0) continue;
-            const double v = nn_val[i];
-            if (v < bv || (v == bv && (bi < 0 || i < bi))) { bv = v; bi = i; }
+    for (int32_t k = 0; k + 1 < n; ++k) {
+        if (tid == 0 && s_len == 0) {                        // an empty chain restarts at the first active slot
+            while (!size[s_first]) ++s_first;
+            chain[0] = s_first; s_len = 1;
         }
-        for (int off = 16; off; off >>= 1) {
-            const double ov = __shfl_down_sync(0xffffffffu, bv, off);
-            const int32_t oi = __shfl_down_sync(0xffffffffu, bi, off);
-            if (oi >= 0 && (bi < 0 || ov < bv || (ov == bv && oi < bi))) { bv = ov; bi = oi; }
-        }
-        if (lane == 0) { s_val[warp] = bv; s_row[warp] = bi; }
-        __syncthreads();
-        if (tid == 0) {
-            double v = s_val[0]; int32_t r = s_row[0];
-            for (int w = 1; w < nwarp; ++w)
-                if (s_row[w] >= 0 && (r < 0 || s_val[w] < v || (s_val[w] == v && s_row[w] < r))) { v = s_val[w]; r = s_row[w]; }
-            const int32_t a = r, b = nn_idx[r];
-            s_a = a; s_b = b; s_ntodo = 0;
-            const int32_t la = label[a], lb = label[b];
-            Z[4 * t + 0] = (double)(la < lb ? la : lb);
-            Z[4 * t + 1] = (double)(la < lb ? lb : la);
-            Z[4 * t + 2] = v;
-            Z[4 * t + 3] = (double)(size[a] + size[b]);
-        }
-        __syncthreads();
-        const int32_t a = s_a, b = s_b;                     // a < b: the merged cluster takes slot a
-        const double sa = (double)size[a], sb = (double)size[b];
-        // (2) distances of the merged cluster, and what they do to the rows' nearest neighbours
-        for (int32_t k = tid; k < n; k += UPGMA_THREADS) {
-            if (!active[k] || k == a || k == b) continue;
-            const double dka = M[(int64_t)k * n + a], dkb = M[(int64_t)k * n + b];
-            const double d = (sa * dka + sb * dkb) / (sa + sb);
-            M[(int64_t)k * n + a] = d;
-            M[(int64_t)a * n + k] = d;
-            if (k < a) {
-                if (nn_idx[k] == a || nn_idx[k] == b) todo[atomicAdd(&s_ntodo, 1)] = k;
-                else if (d < nn_val[k] || (d == nn_val[k] && a < nn_idx[k])) { nn_val[k] = d; nn_idx[k] = a; }
-            } else if (k < b) {
-                if (nn_idx[k] == b) todo[atomicAdd(&s_ntodo, 1)] = k;
+        // walk the chain until its top two are each other's nearest neighbours
+        for (;;) {
+            if (tid == 0) s_x = chain[s_len - 1];
+            __syncthreads();
+            const int32_t x = s_x;
+            const double *row = M + (int64_t)x * n;
+            double bv = 1.0 / 0.0;
+            int32_t bi = 0x7fffffff;
+            for (int32_t i = tid; i < n; i += UPGMA_THREADS)
+                if (i != x && size[i]) upgma_take_min(bv, bi, row[i], i);
+            for (int off = 16; off; off >>= 1)
+                upgma_take_min(bv, bi, __shfl_down_sync(0xffffffffu, bv, off), __shfl_down_sync(0xffffffffu, bi, off));
+            if (lane == 0) { s_val[warp] = bv; s_idx[warp] = bi; }
+            __syncthreads();
+            if (warp == 0) {
+                bv = s_val[lane]; bi = s_idx[lane];
+                for (int off = 16; off; off >>= 1)
+                    upgma_take_min(bv, bi, __shfl_down_sync(0xffffffffu, bv, off), __shfl_down_sync(0xffffffffu, bi, off));
+                if (lane == 0) {
+                    const int32_t prev = s_len > 1 ? chain[s_len - 2] : -1;
+                    if (prev >= 0 && !(bv < row[prev])) {        // the previous element is (one of) the closest: merge
+                        s_y = prev; s_merge = 1;
+                    } else {
+                        chain[s_len++] = bi; s_merge = 0;
+                    }
+                }
             }
+            __syncthreads();
+            if (s_merge) break;
         }
-        __syncthreads();
+        const int32_t x = min(s_x, s_y), y = max(s_x, s_y);
+        const int32_t nx = size[x], ny = size[y];
+        const double fx = (double)nx, fy = (double)ny, fxy = (double)(nx + ny);
         if (tid == 0) {
-            size[a] += size[b]; label[a] = n + t; active[b] = 0;
-            todo[s_ntodo++] = a;
+            Z[4 * (int64_t)k + 0] = (double)x;
+            Z[4 * (int64_t)k + 1] = (double)y;
+            Z[4 * (int64_t)k + 2] = M[(int64_t)x * n + y];
+            Z[4 * (int64_t)k + 3] = fxy;
+        }
+        // the merged cluster replaces y; the reads of rows x and y and the writes of row y are contiguous
+        for (int32_t i = tid; i < n; i += UPGMA_THREADS) {
+            if (i == x || i == y || !size[i]) continue;
+            const double d = __ddiv_rn(__dadd_rn(__dmul_rn(fx, M[(int64_t)x * n + i]), __dmul_rn(fy, M[(int64_t)y * n + i])), fxy);
+            M[(int64_t)y * n + i] = d;
+            M[(int64_t)i * n + y] = d;
         }
         __syncthreads();
-        // (3) rows whose nearest neighbour was merged away (and the merged row itself): full rescan, one warp per row
-        const int32_t nt = s_ntodo;
-        for (int32_t q = warp; q < nt; q += nwarp) upgma_rescan(M, n, active, todo[q], lane, nn_val, nn_idx);
+        if (tid == 0) { size[x] = 0; size[y] = nx + ny; s_len -= 2; }
         __syncthreads();
     }
 }

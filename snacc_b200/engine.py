@@ -206,14 +206,18 @@ class Engine:
         return D
 
     def upgma(self, D, metrify=True):
-        """scipy-style linkage matrix ((n-1) x 4) of average-linkage clustering of the distance matrix D, computed on
-        the device; ``metrify`` first symmetrises D and zeroes its diagonal (reference misc.py:20-25)"""
+        """scipy's linkage matrix ((n-1) x 4) of average-linkage clustering of the distance matrix D, computed on the
+        device; ``metrify`` first symmetrises D and zeroes its diagonal (reference misc.py:20-25).  Raises ValueError
+        where scipy does: a non-finite entry, and with ``metrify`` off an asymmetric matrix or a non-zero diagonal."""
         D = np.ascontiguousarray(D, dtype=np.float64)
-        n = D.shape[0]
+        n = D.shape[0] if D.ndim else 0
         if D.ndim != 2 or D.shape[1] != n or n < 2:
             raise ValueError("D must be a square matrix with at least two rows")
         Z = np.zeros((n - 1, 4), dtype=np.float64)
-        self._check(self._lib.snacc_upgma(self._h, D.ctypes.data, n, int(bool(metrify)), Z.ctypes.data))
+        rc = self._lib.snacc_upgma(self._h, D.ctypes.data, n, int(bool(metrify)), Z.ctypes.data)
+        if rc == -2:                                   # input the reference rejects
+            raise ValueError(self._lib.snacc_last_error(self._h).decode(errors="replace"))
+        self._check(rc)
         return Z
 
     # ---- instrumentation ----
