@@ -104,4 +104,51 @@ void emu_bz2_code_lengths(const int32_t *freq, int32_t alpha_size, int32_t max_l
     bz_make_code_lengths(len, freq, alpha_size, max_len, scratch);
 }
 
+// last column of the sorted cyclic rotations of t[0, n) (the emulator's BWT)
+void emu_bz2_bwt(const uint8_t *t, uint32_t n, uint8_t *L)
+{
+    std::vector<uint8_t> out;
+    host_bwt(t, n, out);
+    std::copy(out.begin(), out.end(), L);
+}
+
+// bits of one block from its last column L[0, n): MTF + RLE2, table choice and bit count, serially
+int64_t emu_bz2_block_bits(const uint8_t *L, uint32_t n)
+{
+    BzWork w;
+    return bz_block_bits_serial(L, n, w);
+}
+
+// how many of the code-length builds of a block's table choice (BZ_N_ITERS iterations x nGroups tables) hit the
+// 17-bit cap and rescaled: the iterations of bz_block_bits_serial, each build repeated without the cap
+int32_t emu_bz2_rescaled_builds(const uint8_t *L, uint32_t n)
+{
+    uint8_t in_use[256] = {0}, seq_of[256], yy[256], len[BZ_N_GROUPS * BZ_MAX_ALPHA], free_len[BZ_MAX_ALPHA];
+    int32_t freq[BZ_MAX_ALPHA], rfreq[BZ_N_GROUPS * BZ_MAX_ALPHA], scratch[BZ_HB_SCRATCH];
+    for (uint32_t i = 0; i < n; ++i) in_use[L[i]] = 1;
+    const int nInUse = bz_map(in_use, seq_of), alphaSize = nInUse + 2;
+    std::vector<uint16_t> mtfv((size_t)n + 1);
+    const uint32_t nMTF = bz_mtf(L, n, seq_of, nInUse, yy, mtfv.data(), freq);
+    const int nGroups = bz_n_groups(nMTF);
+    bz_init_tables(len, nGroups, alphaSize, freq, nMTF);
+    const int nSel = (int)((nMTF + BZ_G_SIZE - 1) / BZ_G_SIZE);
+    int32_t rescaled = 0;
+    for (int iter = 0; iter < BZ_N_ITERS; ++iter) {
+        for (int k = 0; k < BZ_N_GROUPS * BZ_MAX_ALPHA; ++k) rfreq[k] = 0;
+        for (int g = 0; g < nSel; ++g) {
+            const uint32_t gs = (uint32_t)g * BZ_G_SIZE, ge = gs + BZ_G_SIZE - 1 < nMTF ? gs + BZ_G_SIZE - 1 : nMTF - 1;
+            uint32_t c;
+            const int bt = bz_group_choose(len, nGroups, mtfv.data(), gs, ge, &c);
+            for (uint32_t i = gs; i <= ge; ++i) rfreq[bt * BZ_MAX_ALPHA + mtfv[i]]++;
+        }
+        for (int t = 0; t < nGroups; ++t) {
+            bz_make_code_lengths(len + t * BZ_MAX_ALPHA, rfreq + t * BZ_MAX_ALPHA, alphaSize, BZ_MAX_CODE_LEN, scratch);
+            // no code of alphaSize symbols is longer than alphaSize - 1 < BZ_MAX_ALPHA bits: this build never rescales
+            bz_make_code_lengths(free_len, rfreq + t * BZ_MAX_ALPHA, alphaSize, BZ_MAX_ALPHA, scratch);
+            rescaled += *std::max_element(free_len, free_len + alphaSize) > BZ_MAX_CODE_LEN;
+        }
+    }
+    return rescaled;
+}
+
 }  // extern "C"

@@ -1,7 +1,8 @@
 """CPU: the product's bzip2 size functions (snacc_b200/csrc/bzip2.cuh: RLE1, block cut, x-prefix / junction
 decomposition of a pair, MTF + RLE2, Huffman table choice, bit count), compiled for the host by tests/host_emu_bzip2.cu
 with a plain host rotation sort as the BWT, against len(bz2.compress(...)) -- the reference's own call
-(pairwise_ncd.py:76)."""
+(pairwise_ncd.py:76).  Also pins the numpy reference BWT of tests/test_bzip2_kernels_gpu.py to that host sort, and
+checks that its crafted Fibonacci last columns reach the 17-bit code-length cap."""
 import bz2
 import ctypes
 import os
@@ -31,6 +32,10 @@ def bz(tmp_path_factory):
     e.emu_bz2_block_lengths.argtypes = [ctypes.c_char_p, ctypes.c_uint32, ctypes.c_void_p, ctypes.c_int64]
     e.emu_bz2_code_lengths.restype = None
     e.emu_bz2_code_lengths.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p]
+    e.emu_bz2_bwt.restype = None
+    e.emu_bz2_bwt.argtypes = [ctypes.c_char_p, ctypes.c_uint32, ctypes.c_void_p]
+    e.emu_bz2_rescaled_builds.restype = ctypes.c_int32
+    e.emu_bz2_rescaled_builds.argtypes = [ctypes.c_char_p, ctypes.c_uint32]
     return e
 
 
@@ -186,3 +191,31 @@ def test_fuzz_planted_repeats(bz):
             got, _ = pair(bz, s[:cut], s[cut:])
             assert got == len(bz2.compress(s)), (len(s), cut)
         assert single(bz, s) == len(bz2.compress(s))
+
+
+def test_reference_bwt_equals_the_emulator(bz):
+    # the numpy BWT that tests/test_bzip2_kernels_gpu.py holds the device kernels to, pinned byte for byte to the
+    # emulator's on every block those tests use
+    from test_bzip2_kernels_gpu import family_cases, parallel_map, ref_bwt
+
+    def emu_bwt(t):
+        out = ctypes.create_string_buffer(len(t))
+        bz.emu_bz2_bwt(t, len(t), out)
+        return out.raw
+
+    cases = family_cases()
+    bad = [f"{fam} n={n}" for (fam, n, _), a, b in zip(cases, parallel_map(lambda c: ref_bwt(c[2]), cases),
+                                                        parallel_map(lambda c: emu_bwt(c[2]), cases)) if a != b]
+    assert not bad, bad
+
+
+def test_fibonacci_mtf_columns_reach_the_code_length_cap(bz):
+    # the crafted last columns that tests/test_bzip2_kernels_gpu.py gives the bit-count kernel for the 17-bit rescale:
+    # some of their 4 x 6 table builds go past 17 bits and rescale, and not all of them, so the tables' lengths differ
+    from test_bzip2_kernels_gpu import crafted_last_columns
+    cols = crafted_last_columns()
+    for name in ("fibonacci_mtf_25", "fibonacci_mtf_27"):
+        L = cols[name]
+        assert 0 < bz.emu_bz2_rescaled_builds(L, len(L)) < 4 * 6, name
+    # a witness that the count is not positive for any column: random bytes never reach the cap
+    assert bz.emu_bz2_rescaled_builds(cols["nmtf2400"], 2400) == 0
